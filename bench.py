@@ -1,6 +1,7 @@
 """bench.py -- headline benchmark of the MMA hot path (BASELINE.json: "MMA attn fwd+bwd TFLOP/s vs BF16 peak").
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload attn|sft|longctx]
+                    [--dump-outputs DIR]
 
 Workload (config.workload): BASELINE config 3 at the north-star point -- T=8192 context, B=2 per GPU, 32 heads x 96,
 4 interleaved image spans of 128 vision tokens, <|assistant|> 64 tokens before the end, Phi-3 longrope on Q/K,
@@ -59,7 +60,15 @@ def parse():
     ap.add_argument("--no-longctx", action="store_true", help="skip the config-5 section (8K multi-image prefill + decode)")
     ap.add_argument("--no-sft", action="store_true", help="skip the config-4 section (SFT step, DDP when N > 1)")
     ap.add_argument("--prefill-batch", type=int, default=8)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one returned (attention output, LSE, dQ/dK/dV, "
+                         "post-RoPE K) as float32 DIR/<name>.npy, on a fixed sample of token rows")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "attn"):
+        ap.error("--dump-outputs covers the attention workload of --impl ours")
+    return args
 
 
 def init_nccl(dev):
@@ -85,6 +94,24 @@ def make_prompt(B, T, n_img, seed=0):
         lang[:, 8 + k * step] = MEDIA_ID
     lang[:, L - 65] = ASST_ID            # post-splice index T-65 -> q_end = T-64
     return lang, np.ones_like(lang)
+
+
+DUMP_ROWS = 1024    # 1024 token rows x 61.6 KB (o, lse, dq, dk, dv, k_rot in float32) = 63.0 MB per dump
+
+
+def dump_rows(B, T):
+    """The token rows (b * T + t, ascending) --dump-outputs writes: drawn with a fixed seed, the same for the same B and
+    T, so that two builds compare row for row."""
+    return np.sort(np.random.default_rng(0).choice(B * T, size=min(B * T, DUMP_ROWS), replace=False))
+
+
+def dump_outputs(out_dir, B, T, outputs):
+    """Writes each (B, T, ...) array of `outputs`, restricted to the rows of dump_rows(), as float32 out_dir/<name>.npy."""
+    rows = torch.from_numpy(dump_rows(B, T))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, x in outputs.items():
+        sample = x.flatten(0, 1)[rows.to(x.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), sample.float().cpu().numpy())
 
 
 def peaks():
@@ -230,7 +257,8 @@ def prefill_section(dev, rank, world, steps, warmup, longctx=None):
     then 32 greedy decode steps.  LM only: the vision tower is replaced by N(0,0.02) vision tokens (SURVEY 8d).
     e2e: host token ids + host vision tokens -> device -> segments + splice kernels -> prefill -> argmax -> host.
     longctx=(B, T, n_img, n_dec): BASELINE config 5 instead -- n_img x 128 image tokens interleaved in a T-token
-    context (the prompt of the attention benchmark), then n_dec greedy decode steps against the long cache."""
+    context (the prompt of the attention benchmark), then n_dec greedy decode steps against the long cache.
+    Timed: `steps` prefills (resident, then e2e) after max(3, warmup // 3) warm-up prefills of each."""
     import aki_b200
     from aki_b200 import ops
     from aki_b200.model import AkiPhi3Runner, phi35_mini_config
@@ -278,19 +306,21 @@ def prefill_section(dev, rank, world, steps, warmup, longctx=None):
         host_out.copy_(logits[:, -1].argmax(-1), non_blocking=True)
         torch.cuda.current_stream().synchronize()
 
+    from aki_b200._lib import lib as _clib
     res = {}
     for name, fn in (("resident", prefill_resident), ("e2e", prefill_e2e)):
         for _ in range(max(3, warmup // 3)):
             fn()
         barrier()
         a, b_ = ev(), ev()
-        n = max(5, steps // 5)
+        launches0 = _clib.aki_mma_launch_count()
         a.record()
-        for _ in range(n):
+        for _ in range(steps):
             fn()
         b_.record()
+        res[name + "_launches"] = int(_clib.aki_mma_launch_count() - launches0)
         barrier()
-        res[name] = a.elapsed_time(b_) / n
+        res[name] = a.elapsed_time(b_) / steps
     # decode: n_dec steps on top of the last prefill
     logits = prefill_resident()
     tok = logits[:, -1].argmax(-1, keepdim=True)
@@ -329,7 +359,8 @@ def prefill_section(dev, rank, world, steps, warmup, longctx=None):
                         f"({n_img} image(s) x {N} + {L - n_img} text), KV cache written in place, residual + RMSNorm and SiLU gate as fused kernels of this "
                         f"library around cuBLAS GEMMs, last-token logits; "
                         f"{n_dec} greedy decode steps",
-            "prefill_tokens_per_s": world * B * T / (r_ms * 1e-3), "prefill_ms": r_ms,
+            "prefill_tokens_per_s": world * B * T / (r_ms * 1e-3), "prefill_ms": r_ms, "prefill_steps": steps,
+            "prefill_gpu_launches": res["resident_launches"],
             "prefill_e2e_tokens_per_s": world * B * T / (e_ms * 1e-3), "prefill_e2e_ms": e_ms,
             "e2e_h2d_bytes": int(host_ids.numel() * 8 * 2 + host_vis.numel() * 2), "e2e_d2h_bytes": B * 8,
             "decode_tokens_per_s": world * B / (d_ms * 1e-3), "decode_ms_per_step": d_ms,
@@ -605,7 +636,7 @@ def main():
         _clib.aki_mma_set_timing_events(a.cuda_event, b_.cuda_event)
         return a, b_
 
-    def step(timed):
+    def step(timed, keep=None):
         e0, e1, e2 = ev(), ev(), ev()
         e0.record()
         ops.rope_kv_write(qkv, cos, sin, k_rot, None, 0, H)
@@ -617,6 +648,8 @@ def main():
         e2.record()
         if timed:
             per_fwd.append((e0, e1)); per_bwd.append((e1, e2)); per_fwd_k.append(kf); per_bwd_k.append(kb)
+        if keep is not None:
+            keep.update(o=o, lse=lse)
 
     def barrier():
         if world > 1:
@@ -631,9 +664,10 @@ def main():
     sampler.mark_begin()
     t_start, t_end = ev(), ev()
     launches0 = _clib.aki_mma_launch_count()
+    last = {} if args.dump_outputs else None                      # o and lse of the last timed step
     t_start.record()
-    for _ in range(args.steps):
-        step(True)
+    for i in range(args.steps):
+        step(True, last if i == args.steps - 1 else None)
     t_end.record()
     gpu_launches = int(_clib.aki_mma_launch_count() - launches0)      # kernels of libaki_mma.so enqueued in the timed region
     barrier()
@@ -644,6 +678,10 @@ def main():
     bwd_ms = statistics.mean(a.elapsed_time(b) for a, b in per_bwd)
     fwd_k_ms = statistics.mean(a.elapsed_time(b) for a, b in per_fwd_k)
     bwd_k_ms = statistics.mean(a.elapsed_time(b) for a, b in per_bwd_k)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, B, T, {"o": last["o"], "lse": last["lse"].transpose(1, 2), "d_q": dviews[0],
+                                               "d_k": dviews[1], "d_v": dviews[2], "k_rot": k_rot.transpose(1, 2)})
+    del last
 
     # ---- decode attention kernel alone (HBM-bound): B=8 sequences x 32 heads against an 8K-token cache --------
     Bd, Td = 8, 8192
@@ -736,11 +774,11 @@ def main():
     note = lambda m: (sys.stderr.write(f"[bench rank {rank}] {m} t={time.time() - _T0:.1f}s\n"), sys.stderr.flush())
     note("attention + e2e done")
     if not args.no_prefill:
-        prefill = prefill_section(dev, rank, world, args.steps, args.warmup)
+        prefill = prefill_section(dev, rank, world, max(5, args.steps // 5), args.warmup)
     note("prefill section done")
     if not args.no_longctx:
         # BASELINE config 5 at every N of the scaling run: 4 x 128 image tokens in an 8K context, B=2 per GPU, 128 decode steps
-        longctx = prefill_section(dev, rank, world, max(10, args.steps // 2), args.warmup, longctx=(2, 8192, 4, 128))
+        longctx = prefill_section(dev, rank, world, max(5, args.steps // 10), args.warmup, longctx=(2, 8192, 4, 128))
     note("longctx section done")
     if not args.no_sft:
         # BASELINE config 4 at every N of the scaling run: the one workload of the path with a real collective (DDP)

@@ -178,6 +178,20 @@ def test_bench_prompt_geometry():
     assert O.count_allowed(S) == int(O.expand_segments_to_4d(S).sum())
 
 
+def test_bench_rejects_arguments_it_cannot_honour(monkeypatch):
+    """No timed step to report, or an output dump of a path other than the attention step of this library."""
+    sys.path.insert(0, ROOT)
+    import bench
+    for argv in (["--steps", "0"], ["--warmup", "-1"], ["--impl", "reference", "--dump-outputs", "d"],
+                 ["--workload", "sft", "--dump-outputs", "d"]):
+        monkeypatch.setattr(sys, "argv", ["bench.py"] + argv)
+        with pytest.raises(SystemExit):
+            bench.parse()
+    monkeypatch.setattr(sys, "argv", ["bench.py", "--steps", "3", "--dump-outputs", "d"])
+    args = bench.parse()
+    assert args.steps == 3 and args.dump_outputs == "d"
+
+
 def test_bench_reference_arm_prints_exactly_one_json_line():
     """Driver contract: `bench.py --impl reference` runs on the host cores only and prints ONE JSON line on stdout
     (anything native libraries write to fd 1 is diverted to stderr); other ranks of a torchrun launch print nothing."""
