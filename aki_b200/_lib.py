@@ -36,7 +36,7 @@ class AttnParams(C.Structure):
         ("kv_valid_bits", C.c_void_p), ("kv_mutual_bits", C.c_void_p),
         ("q_tile_kv_end", C.c_void_p), ("kv_tile_q_mask", C.c_void_p),
         ("meta_pitch", C.c_int32), ("bits_pitch", C.c_int32),
-        ("fwd_plan", C.c_void_p), ("plan_pairs", C.c_int32), ("reserved0", C.c_int32),
+        ("fwd_plan", C.c_void_p), ("plan_pairs", C.c_int32), ("q_offset", C.c_int32),
     ]
 
 
@@ -58,8 +58,12 @@ _SIGNATURES = {
                                    C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "aki_mma_tile_bounds": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p,
                                       C.c_void_p, C.c_void_p]),
+    "aki_mma_tile_bounds_at": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int,
+                                         C.c_void_p, C.c_void_p, C.c_void_p]),
     "aki_mma_fwd_plan": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int,
                                    C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
+    "aki_mma_fwd_plan_at": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int,
+                                      C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
     "aki_mma_expand_mask": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int,
                                       C.c_int, C.c_void_p, C.c_void_p]),
     "aki_mma_splice": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int,
@@ -80,6 +84,9 @@ _SIGNATURES = {
     "aki_mma_decode": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_void_p,
                                  C.c_int, C.c_int, C.c_int, C.c_int, C.c_float, C.c_void_p, C.c_void_p, C.c_size_t,
                                  C.c_void_p]),
+    "aki_mma_decode_masked": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_void_p,
+                                        C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_float, C.c_void_p,
+                                        C.c_void_p, C.c_size_t, C.c_void_p]),
     "aki_mma_skinny_linear": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_float, C.c_void_p, C.c_int64,
                                         C.c_void_p, C.c_int64, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "aki_mma_add_rmsnorm": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p, C.c_float, C.c_void_p,

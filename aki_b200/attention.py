@@ -25,10 +25,35 @@ import torch
 from torch import nn
 
 from . import ops
-from .cache import AkiKVCache
+from .cache import AkiKVCache, KeyMeta, place_bits
 from .rope import LongRope, half_tables_from_hf
 
 _ctx = threading.local()
+
+
+def _key_valid(attention_mask: Optional[torch.Tensor], n_keys: int) -> Optional[torch.Tensor]:
+    """(B, n_keys) bool validity of the keys of a continuation from HF's mask: 2-D (B, past+T) 0/1, or 4-D
+    (B, 1, T, past+T) reduced to its last query row (bool: True = visible; integer: 1 = visible; floating: additive,
+    0 = visible).  The MMA term of the chunk comes from mma_segments only.  None: every key is valid."""
+    if attention_mask is None:
+        return None
+    m = attention_mask if attention_mask.dim() == 2 else attention_mask[:, 0, -1]
+    m = m[:, :n_keys]
+    if m.dtype == torch.bool:
+        return m
+    return (m == 0) if (attention_mask.dim() == 4 and m.is_floating_point()) else (m != 0)
+
+
+def _foreign_continuation_meta(B: int, t_kv: int, T: int, segs: Optional[ops.MMASegments], attention_mask, device):
+    """Key-coordinate metadata of a continuation onto a cache that keeps no MMA description (DynamicCache, the
+    AttentionInterface plugin): causal over all t_kv keys, validity from the mask, the chunk's own segments shifted."""
+    past = t_kv - T
+    km = KeyMeta(B, t_kv, device)
+    valid = _key_valid(attention_mask, t_kv)
+    if valid is not None and past > 0:
+        place_bits(km.kv_valid_bits, valid[:, :past], 0)
+    km.write_chunk(past, T, segs, None if (segs is not None or valid is None) else valid[:, past:])
+    return km.attn_meta(past, T, segs.max_spans if segs is not None else 8)
 
 
 @contextlib.contextmanager
@@ -103,7 +128,10 @@ class AkiMMAAttention(nn.Module):
         cos, sin = rope
         if segs is not None and hidden_states.shape[1] == 1:
             segs = None          # decode step: the generate loop's mask is all ones (aki_generation.py:56-62)
-        if attention_mask is not None and attention_mask.dim() == 4 and segs is None and hidden_states.shape[1] > 1:
+        continuing = hasattr(past_key_values, "get_seq_length") and past_key_values.get_seq_length(self.layer_idx or 0) > 0
+        if (attention_mask is not None and attention_mask.dim() == 4 and segs is None and hidden_states.shape[1] > 1
+                and not continuing):
+            # (a continuation reduces a 4-D mask to key validity, see _key_valid)
             # (a one-token step gets HF's (B,1,1,T_kv) row, all visible by the generate contract: nothing to describe)
             raise ValueError("a materialised 4-D mask was passed without mma_segments: build the compact description "
                              "with aki_b200.prepare_inputs_for_forward / ops.build_segments instead")
@@ -125,7 +153,7 @@ class AkiMMAAttention(nn.Module):
                 ops.rope_kv_write(qkv, cos, sin, cache.k[self.layer_idx], cache.v[self.layer_idx], 0, H, q_rot=q_rot,
                                   past_len_dev=cache.past_dev)
                 o = ops.decode_op(q_rot.view(B, H, D), cache.k[self.layer_idx], cache.v[self.layer_idx], cache.kv_len,
-                                  cache.t_cap, self.scaling, cache.kv_start).view(B, 1, H * D)
+                                  cache.t_cap, self.scaling, cache.kv_start, cache.meta.kv_valid_bits).view(B, 1, H * D)
                 return self.o_proj(o), None
             past = cache.reserve(self.layer_idx, T)
             if T == 1 and past > 0:
@@ -133,16 +161,28 @@ class AkiMMAAttention(nn.Module):
                 ops.rope_kv_write(qkv, cos, sin, cache.k[self.layer_idx], cache.v[self.layer_idx], past, H, q_rot=q_rot)
                 cache.commit(self.layer_idx, 1)
                 o = ops.decode_op(q_rot.view(B, H, D), cache.k[self.layer_idx], cache.v[self.layer_idx], cache.kv_len,
-                                  past + 1, self.scaling, cache.kv_start).view(B, 1, H * D)
+                                  past + 1, self.scaling, cache.kv_start, cache.meta.kv_valid_bits).view(B, 1, H * D)
+            elif past > 0:
+                # follow-up turn / chunked prefill: the chunk's queries are key rows [past, past + T) of the cache.  The
+                # chunk's mutual intervals come from its own segments (an image row sees the later keys of its chunk up
+                # to that chunk's <|assistant|>: the single-turn rule applied per turn).
+                ops.rope_kv_write(qkv, cos, sin, cache.k[self.layer_idx], cache.v[self.layer_idx], past, H)
+                cache.commit(self.layer_idx, T)
+                valid = None if segs is not None else _key_valid(attention_mask, past + T)
+                meta = cache.chunk_meta(past, T, segs, None if valid is None else valid[:, past:],
+                                        first=self.layer_idx in (0, None))
+                k4 = cache.k[self.layer_idx][:, :, :past + T].transpose(1, 2)
+                v4 = cache.v[self.layer_idx][:, :, :past + T].transpose(1, 2)
+                q4 = qkv[..., : H * D].unflatten(-1, (H, D))
+                o, _ = ops.attn_fwd_raw(q4, k4, v4, cos, sin, meta, self.scaling, need_lse=False, q_offset=past)
+                o = o.view(B, T, H * D)
             else:
-                if past != 0:
-                    raise NotImplementedError("chunked prefill onto a non-empty cache is not part of the reference path "
-                                              "(vision inputs are only spliced at step 0, aki.py:172-207)")
                 ops.rope_kv_write(qkv, cos, sin, cache.k[self.layer_idx], cache.v[self.layer_idx], 0, H)
                 cache.commit(self.layer_idx, T)
                 if self.layer_idx in (0, None):      # decode steps skip the leading pad rows of a left-padded prompt
                     cache.set_key_start(segs.spliced_mask_2d() if segs is not None else
                                         (attention_mask if attention_mask is not None and attention_mask.dim() == 2 else None))
+                    cache.write_prefill_meta(T, segs)
                 k4 = cache.k[self.layer_idx][:, :, :T].transpose(1, 2)
                 v4 = cache.v[self.layer_idx][:, :, :T].transpose(1, 2)
                 q4 = qkv[..., : H * D].unflatten(-1, (H, D))
@@ -165,7 +205,10 @@ class AkiMMAAttention(nn.Module):
                 kv_len = torch.full((B,), t_kv, dtype=torch.int32, device=qkv.device)
                 o = ops.decode_op(q_rot.view(B, H, D), k_all, v_all, kv_len, t_kv, self.scaling).view(B, 1, H * D)
             else:
-                raise NotImplementedError("multi-token continuation onto a non-empty cache")
+                meta = _foreign_continuation_meta(B, t_kv, T, segs, attention_mask, qkv.device)
+                o, _ = ops.attn_fwd_raw(q_rot.transpose(1, 2), k_all.transpose(1, 2), v_all.transpose(1, 2), None, None,
+                                        meta, self.scaling, need_lse=False, q_offset=t_kv - T)
+                o = o.view(B, T, H * D)
         return self.o_proj(o), None
 
 
@@ -183,9 +226,14 @@ def aki_mma_attention(module, query, key, value, attention_mask, scaling: Option
     B, H, T, D = query.shape
     if T == 1:
         segs = None                                 # decode step: all cached keys visible (aki_generation.py:56-62)
+    if key.shape[2] != T and T > 1:
+        # continuation: the queries are the last T of key.shape[2] keys
+        t_kv = key.shape[2]
+        meta = _foreign_continuation_meta(B, t_kv, T, segs, attention_mask, query.device)
+        o, _ = ops.attn_fwd_raw(query.transpose(1, 2), key.transpose(1, 2), value.transpose(1, 2), None, None, meta,
+                                float(scaling), need_lse=False, q_offset=t_kv - T)
+        return o, None
     if key.shape[2] != T:
-        if T != 1:
-            raise NotImplementedError("multi-token continuation onto a non-empty cache")
         kv_len = torch.full((B,), key.shape[2], dtype=torch.int32, device=query.device)
         o = ops.decode_op(query.reshape(B, H, D), key.contiguous(), value.contiguous(), kv_len, key.shape[2], scaling)
         return o.view(B, 1, H, D), None

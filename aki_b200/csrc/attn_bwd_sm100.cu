@@ -833,6 +833,7 @@ using namespace aki;
 extern "C" int aki_mma_attn_bwd(const AkiMmaAttnBwdParams* p, aki_stream_t stream) {
   AKI_REQUIRE(p, AKI_ERR_NULL);
   const AkiMmaAttnParams& f = p->fwd;
+  AKI_REQUIRE(f.q_offset == 0, AKI_ERR_UNSUPPORTED);   // no backward for a continuation chunk
   int rc = check_attn_params(f);
   if (rc) return rc;
   if ((rc = check_tensor(p->d_o)) || (rc = check_tensor(p->d_q)) || (rc = check_tensor(p->d_k)) ||

@@ -79,6 +79,7 @@ struct FwdKernelParams {
   const int4* plan;      // (B, 1 + plan_pairs) or nullptr
   int plan_pairs;
   int B, H, T;
+  int q_off;             // queries are key rows [q_off, q_off + T) (AkiMmaAttnParams.q_offset)
   int ranks, group, n_items, use_clc;   // items: ((g * ranks + r) * group + slice)
   float scale_log2, scale;
   unsigned long long* trace;  // debug build (make TRACE=1, tools/fwd_trace.py): clock64 stamps of one CTA's first item
@@ -279,7 +280,7 @@ attn_fwd_sm100_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_co
     if (lane == 0) {
       uint32_t n_pub = 0, n_clc = 0;
       long long id = blockIdx.x;
-      const int n_kt = (P.T + BN - 1) / BN;
+      const int n_keys = P.q_off + P.T, n_kt = (n_keys + BN - 1) / BN;
       auto publish = [&](const int4& v0, const int4& v1, const int4& v2) {
         const int slot = n_pub % SLOTS;
         mbar_wait(BAR(ITEM_EMPTY + slot), ((n_pub / SLOTS) & 1) ^ 1);
@@ -294,7 +295,7 @@ attn_fwd_sm100_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_co
         const int r = rem / P.group, bh = g * P.group + rem % P.group;
         if (bh < P.B * P.H) {
           const int b = bh / P.H, h = bh % P.H;
-          const int len = meta_len(P.mm, b, P.T);
+          const int len = meta_len(P.mm, b, n_keys);
           int4 e = make_int4(0, 0, 0, 0);
           int first_bad = 0;
           bool ok = false;
@@ -303,7 +304,7 @@ attn_fwd_sm100_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_co
             const int4 hdr = __ldg(row);
             if (r < hdr.x) { e = __ldg(row + 1 + r); first_bad = hdr.y; ok = true; }
           } else {
-            // no plan: aligned tiles (2p, 2p+1), heaviest pair first
+            // no plan: aligned tiles (2p, 2p+1) of the query rows, heaviest pair first
             const int n_qt = (P.T + BM - 1) / BM, p = P.ranks - 1 - r;
             if (p >= 0 && 2 * p < n_qt) {
               ok = true;
@@ -312,19 +313,20 @@ attn_fwd_sm100_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_co
                 int nk = 0, rows = 0;
                 if (qt < n_qt) {
                   rows = min(BM, P.T - qt * BM);
-                  nk = P.mm.q_tile_kv_end ? min(__ldg(P.mm.q_tile_kv_end + (size_t)b * n_qt + qt), n_kt) : min(qt + 1, n_kt);
+                  nk = min(P.mm.q_tile_kv_end ? __ldg(P.mm.q_tile_kv_end + (size_t)b * n_qt + qt)
+                                              : (P.q_off + qt * BM + rows + BN - 1) / BN, n_kt);
                 }
                 if (t == 0) { e.x = qt * BM; e.z = nk | (rows << 16); }
                 else { e.y = (qt < n_qt) ? qt * BM : 0; e.w = nk | (rows << 16); }
               }
               // without a plan nobody scanned the key bit-vectors: every tile is evaluated against the predicate
-              first_bad = (P.mm.seq_len || P.mm.vbits) ? 0 : P.T / BN;
+              first_bad = (P.mm.seq_len || P.mm.vbits) ? 0 : n_keys / BN;
             }
           }
           if (ok) {
             const int nk0 = e.z & 0xffff, nk1 = e.w & 0xffff;
             publish(make_int4(1, b, h, len), make_int4(e.x, e.y, e.z >> 16, e.w >> 16),
-                    make_int4(nk0, nk1, min(first_bad, (e.x + 1) / BN), min(first_bad, (e.y + 1) / BN)));
+                    make_int4(nk0, nk1, min(first_bad, (P.q_off + e.x + 1) / BN), min(first_bad, (P.q_off + e.y + 1) / BN)));
           }
         }
         if (!P.use_clc) {
@@ -456,7 +458,7 @@ attn_fwd_sm100_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_co
       if (!v0.x) break;
       const int b = v0.y, len = v0.w;
       const int nk = t ? v2.y : v2.x, n_full = t ? v2.w : v2.z;
-      const int i = (t ? v1.y : v1.x) + r;        // query index in mask coordinates
+      const int i = P.q_off + (t ? v1.y : v1.x) + r;   // query index in mask (key) coordinates
       const bool row_live = (i < len);
       int row_lo = 0, row_hi = 0;
       if (row_live && P.mm.row_lo && nk > 0) {
@@ -644,7 +646,7 @@ attn_fwd_sm100_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_co
 #pragma unroll 1
       for (int t = 0; t < 2; ++t) {
         const int nk = t ? v2.y : v2.x, rows = t ? v1.w : v1.z;
-        const int i = (t ? v1.y : v1.x) + r;
+        const int ql = (t ? v1.y : v1.x) + r, i = P.q_off + ql;   // query row of q / o / lse, its key coordinate
         mbar_wait(BAR(L_READY + t), n_it & 1);
         const float2 lm = lm_s[t][r];
         if (nk > 0) {
@@ -655,8 +657,8 @@ attn_fwd_sm100_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_co
         // rows with no visible key (batch padding, keys all invalid): zeros (DESIGN.md).  Their maximum never left -inf;
         // the row sum alone does not tell (the polynomial exp2 returns 2^-126, not 0, for a masked score)
         const float inv_l = (nk > 0 && i < len && lm.x > 0.f && lm.y > -INFINITY) ? 1.f / lm.x : 0.f;
-        const bool store_row = (r < rows) && (i < P.T);
-        __nv_bfloat16* orow = P.o.row(b, store_row ? i : 0, h);
+        const bool store_row = (r < rows) && (ql < P.T);
+        __nv_bfloat16* orow = P.o.row(b, store_row ? ql : 0, h);
         // tcgen05.ld is warp-collective (.sync.aligned): load unconditionally, predicate only the global stores
 #pragma unroll 1
         for (int c = 0; c < 3; ++c) {
@@ -678,7 +680,7 @@ attn_fwd_sm100_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_co
           }
         }
         if (P.lse && store_row)
-          P.lse[((size_t)b * P.H + h) * P.T + i] = (inv_l > 0.f) ? (lm.y * P.scale + __logf(lm.x)) : INFINITY;
+          P.lse[((size_t)b * P.H + h) * P.T + ql] = (inv_l > 0.f) ? (lm.y * P.scale + __logf(lm.x)) : INFINITY;
         tc_fence_before();
         mbar_arrive(BAR(O_FREE + t));
       }
@@ -787,8 +789,9 @@ extern "C" int aki_mma_attn_fwd(const AkiMmaAttnParams* p, aki_stream_t stream) 
   AKI_REQUIRE(!p->fwd_plan || p->plan_pairs >= ((p->T + fwd::BM - 1) / fwd::BM + 1) / 2, AKI_ERR_BAD_SHAPE);
   CUtensorMap mq, mk, mv;
   if ((rc = make_tile_map(&mq, p->q, p->B, p->H, p->T, fwd::BM))) return rc;
-  if ((rc = make_tile_map(&mk, p->k, p->B, p->H, p->T, fwd::BN))) return rc;
-  if ((rc = make_tile_map(&mv, p->v, p->B, p->H, p->T, fwd::BN))) return rc;
+  const int n_keys = p->q_offset + p->T;   // check_attn_params: no overflow
+  if ((rc = make_tile_map(&mk, p->k, p->B, p->H, n_keys, fwd::BN))) return rc;
+  if ((rc = make_tile_map(&mv, p->v, p->B, p->H, n_keys, fwd::BN))) return rc;
   FwdKernelParams kp;
   kp.q = view_of(p->q); kp.o = view_of(p->o);
   kp.lse = p->lse; kp.rope_cos = p->rope_cos; kp.rope_sin = p->rope_sin; kp.rope_stride_b = p->rope_stride_b;
@@ -796,6 +799,7 @@ extern "C" int aki_mma_attn_fwd(const AkiMmaAttnParams* p, aki_stream_t stream) 
   kp.plan = reinterpret_cast<const int4*>(p->fwd_plan);
   kp.plan_pairs = p->plan_pairs;
   kp.B = p->B; kp.H = p->H; kp.T = p->T;
+  kp.q_off = p->q_offset;
   const int n_qt = (p->T + fwd::BM - 1) / fwd::BM;
   kp.ranks = p->fwd_plan ? p->plan_pairs : (n_qt + 1) / 2;
   const long long slices = (long long)p->B * p->H;

@@ -5,6 +5,7 @@
 //     the tcgen05 kernels on-device at sizes the CPU oracle cannot reach.  Not a product path.
 //   * bwd_preprocess / dq_finalize: small HBM-bound kernels used by the product backward.
 #include <math.h>
+#include <stdint.h>
 #include "attn_aux.cuh"
 
 namespace aki {
@@ -32,11 +33,12 @@ __device__ __forceinline__ float block_reduce(float v, float* red, bool is_max) 
 __global__ void __launch_bounds__(128)
 attn_fwd_simt_kernel(TensorView q, TensorView k, TensorView v, TensorView o, float* __restrict__ lse,
                      const float* __restrict__ rope_cos, const float* __restrict__ rope_sin, int64_t rope_stride_b,
-                     MaskMeta mm, int T, int H, float scale) {
-  extern __shared__ float sc[];  // T scores
+                     MaskMeta mm, int T, int q_off, int H, float scale) {
+  extern __shared__ float sc[];  // q_off + T scores
   __shared__ float qs[96], red[4];
-  const int i = blockIdx.x, h = blockIdx.y, b = blockIdx.z, tid = threadIdx.x;
-  const int len = meta_len(mm, b, T);
+  // i: query row of q / o / lse / the RoPE tables; ia: its row in key (mask) coordinates
+  const int i = blockIdx.x, ia = q_off + i, h = blockIdx.y, b = blockIdx.z, tid = threadIdx.x;
+  const int len = meta_len(mm, b, q_off + T);
   __nv_bfloat16* orow = o.row(b, i, h);
   if (tid < 96) {
     float x = bf(q.row(b, i, h)[tid]);
@@ -51,11 +53,11 @@ attn_fwd_simt_kernel(TensorView q, TensorView k, TensorView v, TensorView o, flo
     qs[tid] = x;
   }
   __syncthreads();
-  const int row_end = (i < len) ? mma_row_end(mm, b, i, len) : 0;
+  const int row_end = (ia < len) ? mma_row_end(mm, b, ia, len) : 0;
   float mx = -INFINITY;
   for (int j = tid; j < row_end; j += 128) {
     float s = -INFINITY;
-    if (mma_allowed(mm, b, i, j, len)) {
+    if (mma_allowed(mm, b, ia, j, len)) {
       const __nv_bfloat16* kr = k.row(b, j, h);
       float acc = 0.f;
 #pragma unroll 8
@@ -312,6 +314,8 @@ attn_bwd_simt_dkv_kernel(const __nv_bfloat16* __restrict__ q_rot, TensorView k, 
 
 int check_attn_params(const AkiMmaAttnParams& p) {
   if (p.B <= 0 || p.H <= 0 || p.T <= 0 || p.B > 65535 || p.H > 65535) return AKI_ERR_BAD_SHAPE;
+  if (p.q_offset < 0 || (int64_t)p.q_offset + p.T > INT32_MAX) return AKI_ERR_BAD_SHAPE;
+  const int64_t n_keys = (int64_t)p.q_offset + p.T;
   if (p.D != AKI_MMA_HEAD_DIM) return AKI_ERR_UNSUPPORTED;
   int rc;
   if ((rc = check_tensor(p.q)) || (rc = check_tensor(p.k)) || (rc = check_tensor(p.v)) || (rc = check_tensor(p.o)))
@@ -319,8 +323,8 @@ int check_attn_params(const AkiMmaAttnParams& p) {
   if ((p.rope_cos == nullptr) != (p.rope_sin == nullptr)) return AKI_ERR_NULL;
   if (p.rope_cos && (!aligned16(p.rope_cos) || !aligned16(p.rope_sin))) return AKI_ERR_MISALIGNED;
   if ((p.row_lo == nullptr) != (p.row_hi == nullptr)) return AKI_ERR_NULL;
-  if (p.row_lo && p.meta_pitch < p.T) return AKI_ERR_BAD_SHAPE;
-  if ((p.kv_valid_bits || p.kv_mutual_bits) && p.bits_pitch * 32 < p.T) return AKI_ERR_BAD_SHAPE;
+  if (p.row_lo && p.meta_pitch < n_keys) return AKI_ERR_BAD_SHAPE;
+  if ((p.kv_valid_bits || p.kv_mutual_bits) && (int64_t)p.bits_pitch * 32 < n_keys) return AKI_ERR_BAD_SHAPE;
   return AKI_OK;
 }
 
@@ -356,7 +360,7 @@ extern "C" int aki_mma_attn_fwd_simt(const AkiMmaAttnParams* p, aki_stream_t str
   int rc = check_attn_params(*p);
   if (rc) return rc;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  const size_t smem = (size_t)p->T * 4;
+  const size_t smem = ((size_t)p->q_offset + p->T) * 4;
   if (smem > 48 * 1024) {
     if (cudaFuncSetAttribute(attn_fwd_simt_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) !=
         cudaSuccess) {
@@ -366,14 +370,15 @@ extern "C" int aki_mma_attn_fwd_simt(const AkiMmaAttnParams* p, aki_stream_t str
   }
   attn_fwd_simt_kernel<<<dim3(p->T, p->H, p->B), 128, smem, st>>>(view_of(p->q), view_of(p->k), view_of(p->v),
                                                                    view_of(p->o), p->lse, p->rope_cos, p->rope_sin,
-                                                                   p->rope_stride_b, mask_meta_from(*p), p->T, p->H,
-                                                                   p->scale);
+                                                                   p->rope_stride_b, mask_meta_from(*p), p->T,
+                                                                   p->q_offset, p->H, p->scale);
   return check_launch();
 }
 
 extern "C" int aki_mma_attn_bwd_simt(const AkiMmaAttnBwdParams* p, aki_stream_t stream) {
   AKI_REQUIRE(p, AKI_ERR_NULL);
   const AkiMmaAttnParams& f = p->fwd;
+  AKI_REQUIRE(f.q_offset == 0, AKI_ERR_UNSUPPORTED);   // no backward for a continuation chunk
   int rc = check_attn_params(f);
   if (rc) return rc;
   if ((rc = check_tensor(p->d_o)) || (rc = check_tensor(p->d_q)) || (rc = check_tensor(p->d_k)) ||

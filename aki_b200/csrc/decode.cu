@@ -34,8 +34,8 @@ __device__ __forceinline__ uint4 ldg_nc_v4(const void* p) {
 __global__ void __launch_bounds__(DEC_THREADS)
 decode_partial_kernel(const __nv_bfloat16* __restrict__ q, const __nv_bfloat16* __restrict__ k_cache,
                       const __nv_bfloat16* __restrict__ v_cache, int64_t cache_stride_b, int64_t cache_stride_h,
-                      const int32_t* __restrict__ kv_len, const int32_t* __restrict__ kv_start, int H, float scale_log2,
-                      int n_splits,
+                      const int32_t* __restrict__ kv_len, const int32_t* __restrict__ kv_start,
+                      const uint32_t* __restrict__ kv_valid_bits, int bits_pitch, int H, float scale_log2, int n_splits,
                       float* __restrict__ ws_m, float* __restrict__ ws_l, float* __restrict__ ws_acc) {
   const int split = blockIdx.x, h = blockIdx.y, b = blockIdx.z;
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, g = lane >> 2, s = lane & 3;
@@ -46,6 +46,8 @@ decode_partial_kernel(const __nv_bfloat16* __restrict__ q, const __nv_bfloat16* 
   // rows at the front of the cache
   const int j0 = max(split * DEC_CHUNK, kv_start ? kv_start[b] : 0), j1 = min(split * DEC_CHUNK + DEC_CHUNK, len);
   const size_t part = ((size_t)b * H + h) * n_splits + split;
+  // interior invalid rows (the left padding of a follow-up turn's prompt): one bit per key
+  const uint32_t* vbits = kv_valid_bits ? kv_valid_bits + (size_t)b * bits_pitch : nullptr;
 
   float qf[24];
   {
@@ -77,6 +79,14 @@ decode_partial_kernel(const __nv_bfloat16* __restrict__ q, const __nv_bfloat16* 
       for (int i = 0; i < 3; ++i) {
         ku[u][i] = ldg_nc_v4(kb + (size_t)jj * DEC_D + (s + 4 * i) * 8);
         vu[u][i] = ldg_nc_v4(vb + (size_t)jj * DEC_D + (s + 4 * i) * 8);
+      }
+    }
+    // the validity bit is folded in after the K / V loads are issued: their addresses must not wait on it
+    if (vbits) {
+#pragma unroll
+      for (int u = 0; u < 2; ++u) {
+        const int j = jb + u * (DEC_THREADS / 32) * 8 + g;
+        if (ok[u]) ok[u] = (__ldg(vbits + (j >> 5)) >> (j & 31)) & 1u;
       }
     }
 #pragma unroll
@@ -174,12 +184,14 @@ extern "C" size_t aki_mma_decode_workspace_bytes(int B, int H, int D, int max_kv
   return (size_t)B * H * splits * (DEC_D + 2) * sizeof(float);
 }
 
-extern "C" int aki_mma_decode(const void* q, const void* k_cache, const void* v_cache, int64_t cache_stride_b,
-                              int64_t cache_stride_h, const int32_t* kv_len, const int32_t* kv_start, int max_kv_len,
-                              int B, int H, int D, float scale, void* out, void* workspace, size_t workspace_bytes,
-                              aki_stream_t stream) {
+extern "C" int aki_mma_decode_masked(const void* q, const void* k_cache, const void* v_cache, int64_t cache_stride_b,
+                                     int64_t cache_stride_h, const int32_t* kv_len, const int32_t* kv_start,
+                                     const uint32_t* kv_valid_bits, int bits_pitch, int max_kv_len, int B, int H, int D,
+                                     float scale, void* out, void* workspace, size_t workspace_bytes,
+                                     aki_stream_t stream) {
   AKI_REQUIRE(q && k_cache && v_cache && kv_len && out && workspace, AKI_ERR_NULL);
   AKI_REQUIRE(B > 0 && H > 0 && max_kv_len > 0 && B <= 65535 && H <= 65535, AKI_ERR_BAD_SHAPE);
+  AKI_REQUIRE(!kv_valid_bits || (long long)bits_pitch * 32 >= max_kv_len, AKI_ERR_BAD_SHAPE);
   AKI_REQUIRE(D == DEC_D, AKI_ERR_UNSUPPORTED);
   AKI_REQUIRE(cache_stride_b % 8 == 0 && cache_stride_h % 8 == 0, AKI_ERR_UNSUPPORTED);
   AKI_REQUIRE(aligned16(q) && aligned16(k_cache) && aligned16(v_cache) && aligned16(workspace), AKI_ERR_MISALIGNED);
@@ -192,11 +204,19 @@ extern "C" int aki_mma_decode(const void* q, const void* k_cache, const void* v_
   const float scale_log2 = scale * 1.4426950408889634f;
   launch_pdl(decode_partial_kernel, dim3(n_splits, H, B), dim3(DEC_THREADS), 0, st,
              static_cast<const __nv_bfloat16*>(q), static_cast<const __nv_bfloat16*>(k_cache),
-             static_cast<const __nv_bfloat16*>(v_cache), cache_stride_b, cache_stride_h, kv_len, kv_start, H, scale_log2,
-             n_splits, ws_m, ws_l, ws_acc);
+             static_cast<const __nv_bfloat16*>(v_cache), cache_stride_b, cache_stride_h, kv_len, kv_start, kv_valid_bits,
+             bits_pitch, H, scale_log2, n_splits, ws_m, ws_l, ws_acc);
   int rc = check_launch();
   if (rc != AKI_OK) return rc;
   launch_pdl(decode_combine_kernel, dim3(H, B), dim3(DEC_D), 0, st, ws_m, ws_l, ws_acc, H, n_splits,
              static_cast<__nv_bfloat16*>(out));
   return check_launch();
+}
+
+extern "C" int aki_mma_decode(const void* q, const void* k_cache, const void* v_cache, int64_t cache_stride_b,
+                              int64_t cache_stride_h, const int32_t* kv_len, const int32_t* kv_start, int max_kv_len,
+                              int B, int H, int D, float scale, void* out, void* workspace, size_t workspace_bytes,
+                              aki_stream_t stream) {
+  return aki_mma_decode_masked(q, k_cache, v_cache, cache_stride_b, cache_stride_h, kv_len, kv_start, nullptr, 0,
+                               max_kv_len, B, H, D, scale, out, workspace, workspace_bytes, stream);
 }

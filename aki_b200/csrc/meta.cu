@@ -138,10 +138,10 @@ segments_kernel(const int64_t* __restrict__ lang_x, const int64_t* __restrict__ 
 
 __global__ void __launch_bounds__(128)
 tile_bounds_kernel(const int32_t* __restrict__ seq_len, const int32_t* __restrict__ row_lo,
-                   const int32_t* __restrict__ row_hi, int T, int t_cap, int n_tiles, int n_words,
+                   const int32_t* __restrict__ row_hi, int T, int q_off, int t_cap, int n_tiles, int n_words,
                    int32_t* __restrict__ q_tile_kv_end, uint32_t* __restrict__ kv_tile_q_mask) {
   const int tile = blockIdx.x, b = blockIdx.y, tid = threadIdx.x;
-  const int len = min(seq_len[b], T);
+  const int len = min(seq_len[b], q_off + T);     // key coordinates; the query rows are [q_off, q_off + T)
   const int32_t* lo = row_lo + (size_t)b * t_cap;
   const int32_t* hi = row_hi + (size_t)b * t_cap;
   __shared__ int s_max;
@@ -152,15 +152,15 @@ tile_bounds_kernel(const int32_t* __restrict__ seq_len, const int32_t* __restric
   const int r0 = tile * AKI_MMA_TILE;
   // query tile: how far right do its rows look
   int need = 0;
-  const int i = r0 + tid;
+  const int i = q_off + r0 + tid;
   if (i < len) {
     need = i + 1;
     const int a = lo[i], e = hi[i];
     if (e > a) need = max(need, min(e, len));
   }
   atomicMax(&s_max, need);
-  // key tile: which query tiles hold a row that sees any of its keys
-  if (r0 < len) {
+  // key tile: which query tiles hold a row that sees any of its keys (q_off == 0: the host refuses the mask otherwise)
+  if (kv_tile_q_mask && r0 < len) {
     const int j1 = min(r0 + AKI_MMA_TILE, len);
     const int n_live = (len + AKI_MMA_TILE - 1) / AKI_MMA_TILE;
     for (int qt = tile + tid; qt < n_live; qt += 128) atomicOr(&s_mask[qt >> 5], 1u << (qt & 31));  // causal part
@@ -185,10 +185,13 @@ constexpr int PLAN_MAX_CUTS = 256;
 
 __global__ void __launch_bounds__(PLAN_THREADS)
 fwd_plan_kernel(const int32_t* __restrict__ seq_len, const int32_t* __restrict__ row_lo,
-                const int32_t* __restrict__ row_hi, const uint32_t* __restrict__ vbits, int T, int meta_pitch,
-                int bits_pitch, int max_pairs, int flags, int4* __restrict__ plan) {
+                const int32_t* __restrict__ row_hi, const uint32_t* __restrict__ vbits, int T, int q_off,
+                int meta_pitch, int bits_pitch, int max_pairs, int flags, int4* __restrict__ plan) {
+  // Rows are in key coordinates throughout: the query rows are [q_off, q_off + T) of q_off + T keys; the plan stores
+  // tile starts relative to q_off.
   const int b = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const int len = seq_len ? min(seq_len[b], T) : T;
+  const int n_keys = q_off + T;
+  const int len = seq_len ? min(seq_len[b], n_keys) : n_keys;
   const int32_t* lo = row_lo ? row_lo + (size_t)b * meta_pitch : nullptr;
   const int32_t* hi = row_hi ? row_hi + (size_t)b * meta_pitch : nullptr;
   __shared__ int s_first_bad, s_ncut, s_ntiles;
@@ -197,7 +200,7 @@ fwd_plan_kernel(const int32_t* __restrict__ seq_len, const int32_t* __restrict__
   __shared__ int s_seg_tile0[PLAN_MAX_CUTS + 2];
   __shared__ int s_start[PLAN_MAX_TILES], s_rows[PLAN_MAX_TILES], s_nkv[PLAN_MAX_TILES];
   __shared__ uint16_t s_order[PLAN_MAX_TILES];
-  const int n_kt = (T + AKI_MMA_TILE - 1) / AKI_MMA_TILE;
+  const int n_kt = (n_keys + AKI_MMA_TILE - 1) / AKI_MMA_TILE;
   if (tid == 0) { s_first_bad = n_kt; s_ncut = 0; }
   __syncthreads();
   // first 128-key tile that is not entirely inside the sequence and causally valid
@@ -211,10 +214,10 @@ fwd_plan_kernel(const int32_t* __restrict__ seq_len, const int32_t* __restrict__
   }
   // change points of the rows' mutual interval: a span STARTS where a row with a non-empty interval follows a row with
   // a different (or no) interval, and ENDS where a row without one follows
-  const int n_aligned = n_kt;
+  const int n_aligned = (T + AKI_MMA_TILE - 1) / AKI_MMA_TILE;
   const int budget = min(max(2 * max_pairs - n_aligned - 1, 0), PLAN_MAX_CUTS);
   if ((flags & 1) && lo && budget > 0) {
-    for (int i = 1 + tid; i < len; i += PLAN_THREADS) {
+    for (int i = q_off + 1 + tid; i < len; i += PLAN_THREADS) {
       const int a = lo[i], e = hi[i], a0 = lo[i - 1], e0 = hi[i - 1];
       const int id = (e > a) ? a : -1, id0 = (e0 > a0) ? a0 : -1;     // identity of the span a row belongs to
       if (id != id0) {
@@ -239,8 +242,18 @@ fwd_plan_kernel(const int32_t* __restrict__ seq_len, const int32_t* __restrict__
     // the following tiles off the 128-key grid (each then straddles one more key tile on its diagonal); cutting again
     // at the next multiple of 128 behind the span puts them back.  Each cut is taken only when the key-tile visits it
     // adds (unused rows of a short tile x the key tiles that tile visits) are fewer than those it saves.
-    int nb = 0, prev = 0;                      // boundaries so far (excluding 0), last boundary
-    s_cut_sorted[0] = 0;
+    int nb = 0, prev = q_off;                  // boundaries so far (excluding q_off), last boundary
+    s_cut_sorted[0] = q_off;
+    if ((flags & 1) && prev % AKI_MMA_TILE != 0 && nb < budget) {
+      // a continuation chunk that starts off the key-tile grid: a short first tile puts the following ones back on it
+      const int G = (prev + AKI_MMA_TILE - 1) / AKI_MMA_TILE * AKI_MMA_TILE;
+      const int next_chg = (nchg > 0) ? s_seg_tile0[0] : len;
+      if (G < next_chg && G < len) {
+        const int waste_realign = (AKI_MMA_TILE - (G - prev)) * (G / AKI_MMA_TILE);   // x 1/128, as below
+        const int waste_stay = min(next_chg, len) - G;
+        if (waste_realign < waste_stay) { s_cut_sorted[++nb] = G; prev = G; }
+      }
+    }
     for (int k = 0; k < nchg && nb < budget; ++k) {
       const int c = s_seg_tile0[k];
       const int a = lo[c], e = hi[c];
@@ -263,7 +276,7 @@ fwd_plan_kernel(const int32_t* __restrict__ seq_len, const int32_t* __restrict__
       }
     }
     s_ncut = nb;
-    s_cut_sorted[1 + nb] = T;
+    s_cut_sorted[1 + nb] = n_keys;
     int n = 0;
     for (int k = 0; k <= nb; ++k) {
       s_seg_tile0[k] = n;
@@ -325,10 +338,10 @@ fwd_plan_kernel(const int32_t* __restrict__ seq_len, const int32_t* __restrict__
     int4 e = make_int4(0, 0, 0, 0);
     if (p < n_pairs) {
       const int x0 = s_order[2 * p];
-      e.x = s_start[x0]; e.z = s_nkv[x0] | (s_rows[x0] << 16);
+      e.x = s_start[x0] - q_off; e.z = s_nkv[x0] | (s_rows[x0] << 16);
       if (2 * p + 1 < n_tiles) {
         const int x1 = s_order[2 * p + 1];
-        e.y = s_start[x1]; e.w = s_nkv[x1] | (s_rows[x1] << 16);
+        e.y = s_start[x1] - q_off; e.w = s_nkv[x1] | (s_rows[x1] << 16);
       }
     }
     out[1 + p] = e;
@@ -396,33 +409,50 @@ extern "C" int aki_mma_segments(const int64_t* lang_x, const int64_t* attention_
   return check_launch();
 }
 
-extern "C" int aki_mma_tile_bounds(const int32_t* seq_len, const int32_t* row_lo, const int32_t* row_hi, int B, int T,
-                                   int t_cap, int32_t* q_tile_kv_end, uint32_t* kv_tile_q_mask, aki_stream_t stream) {
+extern "C" int aki_mma_tile_bounds_at(const int32_t* seq_len, const int32_t* row_lo, const int32_t* row_hi, int B,
+                                      int T, int q_offset, int t_cap, int32_t* q_tile_kv_end, uint32_t* kv_tile_q_mask,
+                                      aki_stream_t stream) {
   AKI_REQUIRE(seq_len && row_lo && row_hi, AKI_ERR_NULL);
-  AKI_REQUIRE(B > 0 && T > 0 && t_cap >= T, AKI_ERR_BAD_SHAPE);
+  AKI_REQUIRE(B > 0 && T > 0 && q_offset >= 0 && (long long)q_offset + T <= INT_MAX, AKI_ERR_BAD_SHAPE);
+  AKI_REQUIRE(t_cap >= q_offset + T, AKI_ERR_BAD_SHAPE);
+  AKI_REQUIRE(q_offset == 0 || !kv_tile_q_mask, AKI_ERR_UNSUPPORTED);   // backward-only data: no continuation backward
   const int n_tiles = (T + AKI_MMA_TILE - 1) / AKI_MMA_TILE;
   const int n_words = (n_tiles + 31) / 32;
   AKI_REQUIRE(n_words <= 64, AKI_ERR_UNSUPPORTED);
   tile_bounds_kernel<<<dim3(n_tiles, B), 128, 0, static_cast<cudaStream_t>(stream)>>>(
-      seq_len, row_lo, row_hi, T, t_cap, n_tiles, n_words, q_tile_kv_end, kv_tile_q_mask);
+      seq_len, row_lo, row_hi, T, q_offset, t_cap, n_tiles, n_words, q_tile_kv_end, kv_tile_q_mask);
+  return check_launch();
+}
+
+extern "C" int aki_mma_tile_bounds(const int32_t* seq_len, const int32_t* row_lo, const int32_t* row_hi, int B, int T,
+                                   int t_cap, int32_t* q_tile_kv_end, uint32_t* kv_tile_q_mask, aki_stream_t stream) {
+  return aki_mma_tile_bounds_at(seq_len, row_lo, row_hi, B, T, 0, t_cap, q_tile_kv_end, kv_tile_q_mask, stream);
+}
+
+extern "C" int aki_mma_fwd_plan_at(const int32_t* seq_len, const int32_t* row_lo, const int32_t* row_hi,
+                                   const uint32_t* kv_valid_bits, int B, int T, int q_offset, int meta_pitch,
+                                   int bits_pitch, int max_pairs, int flags, int32_t* plan, aki_stream_t stream) {
+  AKI_REQUIRE(plan, AKI_ERR_NULL);
+  AKI_REQUIRE((row_lo == nullptr) == (row_hi == nullptr), AKI_ERR_NULL);
+  AKI_REQUIRE(B > 0 && T > 0 && q_offset >= 0 && (long long)q_offset + T <= INT_MAX, AKI_ERR_BAD_SHAPE);
+  const int n_keys = q_offset + T;
+  const int n_aligned = (T + AKI_MMA_TILE - 1) / AKI_MMA_TILE;
+  AKI_REQUIRE(max_pairs >= (n_aligned + 1) / 2, AKI_ERR_BAD_SHAPE);
+  AKI_REQUIRE(2 * max_pairs <= PLAN_MAX_TILES, AKI_ERR_UNSUPPORTED);
+  AKI_REQUIRE(!row_lo || meta_pitch >= n_keys, AKI_ERR_BAD_SHAPE);
+  AKI_REQUIRE(!kv_valid_bits || (long long)bits_pitch * 32 >= n_keys, AKI_ERR_BAD_SHAPE);
+  AKI_REQUIRE(aligned16(plan), AKI_ERR_MISALIGNED);
+  fwd_plan_kernel<<<B, PLAN_THREADS, 0, static_cast<cudaStream_t>(stream)>>>(
+      seq_len, row_lo, row_hi, kv_valid_bits, T, q_offset, meta_pitch, bits_pitch, max_pairs, flags,
+      reinterpret_cast<int4*>(plan));
   return check_launch();
 }
 
 extern "C" int aki_mma_fwd_plan(const int32_t* seq_len, const int32_t* row_lo, const int32_t* row_hi,
                                 const uint32_t* kv_valid_bits, int B, int T, int meta_pitch, int bits_pitch,
                                 int max_pairs, int flags, int32_t* plan, aki_stream_t stream) {
-  AKI_REQUIRE(plan, AKI_ERR_NULL);
-  AKI_REQUIRE((row_lo == nullptr) == (row_hi == nullptr), AKI_ERR_NULL);
-  AKI_REQUIRE(B > 0 && T > 0, AKI_ERR_BAD_SHAPE);
-  const int n_aligned = (T + AKI_MMA_TILE - 1) / AKI_MMA_TILE;
-  AKI_REQUIRE(max_pairs >= (n_aligned + 1) / 2, AKI_ERR_BAD_SHAPE);
-  AKI_REQUIRE(2 * max_pairs <= PLAN_MAX_TILES, AKI_ERR_UNSUPPORTED);
-  AKI_REQUIRE(!row_lo || meta_pitch >= T, AKI_ERR_BAD_SHAPE);
-  AKI_REQUIRE(!kv_valid_bits || bits_pitch >= (T + 31) / 32, AKI_ERR_BAD_SHAPE);
-  AKI_REQUIRE(aligned16(plan), AKI_ERR_MISALIGNED);
-  fwd_plan_kernel<<<B, PLAN_THREADS, 0, static_cast<cudaStream_t>(stream)>>>(
-      seq_len, row_lo, row_hi, kv_valid_bits, T, meta_pitch, bits_pitch, max_pairs, flags, reinterpret_cast<int4*>(plan));
-  return check_launch();
+  return aki_mma_fwd_plan_at(seq_len, row_lo, row_hi, kv_valid_bits, B, T, 0, meta_pitch, bits_pitch, max_pairs, flags,
+                             plan, stream);
 }
 
 extern "C" int aki_mma_expand_mask(const int32_t* seq_len, const int32_t* row_lo, const int32_t* row_hi,

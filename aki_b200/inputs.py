@@ -37,13 +37,19 @@ def prepare_inputs_for_forward(self, vision_tokens: Optional[torch.Tensor], lang
     lang_embeds = self.lang_model.get_input_embeddings()(lang_x)                           # vlm.py:478
     B, L = lang_x.shape
     t_cap = L + vision_tokens.shape[1] * (N - 1)
-    segs = ops.build_segments(lang_x, attention_mask, N, int(self.media_token_id), assistant_token_id, t_cap=t_cap,
-                              text_only=text_only, exact_shape=exact_shape)
+    # a continuation (follow-up turn) describes its own tokens: the mask's last L columns; the cached rows keep theirs
+    past_mask = attention_mask[:, :attention_mask.shape[1] - L] if past_key_values is not None else None
+    segs = ops.build_segments(lang_x, attention_mask[:, -L:] if past_mask is not None else attention_mask, N,
+                              int(self.media_token_id), assistant_token_id, t_cap=t_cap, text_only=text_only,
+                              exact_shape=exact_shape)
     embeds, new_labels = ops.splice(lang_embeds.to(torch.bfloat16), vision_tokens, labels, segs,
                                     pad_value=float(self.pad_token_id), padding_side=padding_side)
     if torch.is_grad_enabled() and padding_side == "right" and (
             lang_embeds.requires_grad or (vision_tokens is not None and vision_tokens.requires_grad)):
         # training: same values, but with the scatter-add backward so that the embedding table / vision side train
         embeds = ops.splice_trainable(lang_embeds.to(torch.bfloat16), vision_tokens, segs, float(self.pad_token_id))
-    return {"inputs_embeds": embeds.to(lang_embeds.dtype), "attention_mask": segs.spliced_mask_2d(),
+    mask = segs.spliced_mask_2d()
+    if past_mask is not None:                 # HF's contract: the 2-D mask covers past + new tokens
+        mask = torch.cat([past_mask.to(mask.dtype), mask], 1)
+    return {"inputs_embeds": embeds.to(lang_embeds.dtype), "attention_mask": mask,
             "labels": new_labels, "mma_segments": segs}

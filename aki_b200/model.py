@@ -81,9 +81,13 @@ class AkiPhi3Runner(nn.Module):
     def prefill(self, inputs_embeds: torch.Tensor, segs: Optional[ops.MMASegments], cache: Optional[AkiKVCache],
                 last_only: bool = True, fused: bool = True):
         """inputs_embeds (B,T,3072); positions arange(T) as AKI.generate passes them (aki.py:184-191).  fused=False runs
-        HF's Phi3DecoderLayer objects (the parity reference of the fused pass)."""
+        HF's Phi3DecoderLayer objects (the parity reference of the fused pass).  Onto a non-empty cache (follow-up turn,
+        chunked prefill) the chunk takes positions past + arange(T), the same for every sequence, with the longrope
+        factor set of the running maximum past + T - 1 (the rule of the decode steps); `segs` then describes the chunk
+        alone (chunk-relative, e.g. build_segments on the chunk's own tokens)."""
         B, T, _ = inputs_embeds.shape
-        cos, sin = self.rope.tables(torch.arange(T, device=inputs_embeds.device)[None], max_position=T - 1)
+        past = cache.get_seq_length() if cache is not None else 0
+        cos, sin = self.rope.tables(past + torch.arange(T, device=inputs_embeds.device)[None], max_position=past + T - 1)
         fused = fused and inputs_embeds.dtype == torch.bfloat16 and inputs_embeds.shape[-1] <= 4096
         h = (self._run_layers_fused if fused else self._run_layers)(inputs_embeds.contiguous() if fused else inputs_embeds,
                                                                       cos, sin, segs, cache)
@@ -119,7 +123,8 @@ class AkiPhi3Runner(nn.Module):
             else:
                 ops.rope_kv_write(qkv.view(B, 1, -1), cos, sin, cache.k[li], cache.v[li], past, H, q_rot=q_rot)
                 max_kv = past + 1
-            o = ops.decode_op(q_rot.view(B, H, D), cache.k[li], cache.v[li], cache.kv_len, max_kv, attn.scaling, cache.kv_start)
+            o = ops.decode_op(q_rot.view(B, H, D), cache.k[li], cache.v[li], cache.kv_len, max_kv, attn.scaling, cache.kv_start,
+                              cache.meta.kv_valid_bits)
             h = ops.skinny_linear(o.view(B, H * D), attn.o_proj.weight, residual=h)
             act = ops.skinny_linear(h, layer.mlp.gate_up_proj.weight, layer.post_attention_layernorm.weight, eps, swiglu=True)
             h = ops.skinny_linear(act, layer.mlp.down_proj.weight, residual=h)
@@ -215,9 +220,12 @@ class AkiPhi3Runner(nn.Module):
         return g["next"].clone()
 
     @torch.no_grad()
-    def generate(self, inputs_embeds, segs, max_new_tokens: int, t_cap: Optional[int] = None):
+    def generate(self, inputs_embeds, segs, max_new_tokens: int, t_cap: Optional[int] = None,
+                 cache: Optional[AkiKVCache] = None):
+        """Greedy generation; with `cache` the prompt is a follow-up turn appended to that cache's contents."""
         B, T, _ = inputs_embeds.shape
-        cache = self.new_cache(B, t_cap or (T + max_new_tokens))
+        if cache is None:
+            cache = self.new_cache(B, t_cap or (T + max_new_tokens))
         logits = self.prefill(inputs_embeds, segs, cache)
         out = []
         tok = logits[:, -1].argmax(-1, keepdim=True)

@@ -108,18 +108,40 @@ def rebuild_tile_bounds(s: MMASegments) -> MMASegments:
 PLAN_FLAGS = int(os.environ.get("AKI_MMA_PLAN_FLAGS", "3"))   # tools only: bit 0 cut at span starts, bit 1 rank + pair
 
 
-def build_fwd_plan(seq_len, row_lo, row_hi, vbits, T: int, max_spans: int = 8, flags: Optional[int] = None) -> torch.Tensor:
-    """Forward work plan (include/aki_mma.h, aki_mma_fwd_plan): (B, 1 + pairs, 4) int32."""
+def build_fwd_plan(seq_len, row_lo, row_hi, vbits, T: int, max_spans: int = 8, flags: Optional[int] = None,
+                   q_offset: int = 0) -> torch.Tensor:
+    """Forward work plan (include/aki_mma.h, aki_mma_fwd_plan_at): (B, 1 + pairs, 4) int32 for the T query rows
+    [q_offset, q_offset + T) of metadata in key coordinates."""
     if not hasattr(lib, "aki_mma_fwd_plan"):      # AKI_MMA_LIB_COMPAT (tools): an ABI-1 build has no plan
         return None
     B = seq_len.shape[0]
     nt = (T + TILE - 1) // TILE
     pairs = (nt + max_spans + 2) // 2
     plan = torch.empty(B, 1 + pairs, 4, dtype=torch.int32, device=seq_len.device)
-    check(lib.aki_mma_fwd_plan(_ptr(seq_len), _ptr(row_lo), _ptr(row_hi), _ptr(vbits), B, T,
-                               row_lo.shape[1] if row_lo is not None else 0, vbits.shape[1] if vbits is not None else 0,
-                               pairs, PLAN_FLAGS if flags is None else flags, _ptr(plan), _stream()), "aki_mma_fwd_plan")
+    mp, bp = (row_lo.shape[1] if row_lo is not None else 0), (vbits.shape[1] if vbits is not None else 0)
+    fl = PLAN_FLAGS if flags is None else flags
+    if q_offset:
+        check(lib.aki_mma_fwd_plan_at(_ptr(seq_len), _ptr(row_lo), _ptr(row_hi), _ptr(vbits), B, T, int(q_offset), mp, bp,
+                                      pairs, fl, _ptr(plan), _stream()), "aki_mma_fwd_plan_at")
+    else:
+        check(lib.aki_mma_fwd_plan(_ptr(seq_len), _ptr(row_lo), _ptr(row_hi), _ptr(vbits), B, T, mp, bp, pairs, fl,
+                                   _ptr(plan), _stream()), "aki_mma_fwd_plan")
     return plan
+
+
+def continuation_meta(seq_len, row_lo, row_hi, vbits, mbits, T: int, q_offset: int, max_spans: int = 8,
+                      plan: bool = True):
+    """Metadata tuple (see meta_tuple) for attn_fwd_raw(..., q_offset=q_offset) from key-coordinate arrays
+    (row_lo / row_hi (B, >= q_offset + T), bits (B, >= ceil((q_offset + T)/32))).  plan=False: per-query-tile key ends
+    (aki_mma_tile_bounds_at) and aligned tiles instead of the work plan."""
+    if plan:
+        return (seq_len, row_lo, row_hi, vbits, mbits, None, None,
+                build_fwd_plan(seq_len, row_lo, row_hi, vbits, T, max_spans, q_offset=q_offset))
+    nt = (T + TILE - 1) // TILE
+    kv_end = torch.empty(seq_len.shape[0], nt, dtype=torch.int32, device=seq_len.device)
+    check(lib.aki_mma_tile_bounds_at(_ptr(seq_len), _ptr(row_lo), _ptr(row_hi), seq_len.shape[0], T, int(q_offset),
+                                     row_lo.shape[1], _ptr(kv_end), None, _stream()), "aki_mma_tile_bounds_at")
+    return (seq_len, row_lo, row_hi, vbits, mbits, kv_end, None, None)
 
 
 def build_segments(lang_x: torch.Tensor, attention_mask: torch.Tensor, num_tokens_per_vis: int, media_token_id: int,
@@ -273,9 +295,11 @@ def _t4(t: torch.Tensor) -> Tensor4:
     return Tensor4(t.data_ptr(), t.stride(0), t.stride(1), t.stride(2))
 
 
-def _fill_params(p: AttnParams, q, k, v, o, lse, cos, sin, meta, scale):
+def _fill_params(p: AttnParams, q, k, v, o, lse, cos, sin, meta, scale, q_offset=0):
     B, T, H, D = q.shape
+    assert k.shape[1] >= q_offset + T and v.shape[1] >= q_offset + T, (k.shape, q.shape, q_offset)
     p.B, p.H, p.T, p.D = B, H, T, D
+    p.q_offset = int(q_offset)
     p.scale = float(scale)
     p.q, p.k, p.v, p.o = _t4(q), _t4(k), _t4(v), _t4(o)
     p.lse = _ptr(lse)
@@ -296,7 +320,7 @@ def _fill_params(p: AttnParams, q, k, v, o, lse, cos, sin, meta, scale):
         p.meta_pitch = row_lo.shape[1] if row_lo is not None else 0
         p.bits_pitch = vbits.shape[1] if vbits is not None else 0
         if row_lo is not None:
-            assert row_lo.shape[1] >= T and row_lo.is_contiguous() and row_hi.is_contiguous()
+            assert row_lo.shape[1] >= q_offset + T and row_lo.is_contiguous() and row_hi.is_contiguous()
         if qkv_end is not None:
             assert qkv_end.shape[1] == (T + TILE - 1) // TILE and qkv_end.is_contiguous()
 
@@ -308,14 +332,16 @@ def meta_tuple(segs: Optional[MMASegments]):
             segs.kv_tile_q_mask, segs.fwd_plan)
 
 
-def attn_fwd_raw(q, k, v, cos, sin, meta, scale, need_lse=True, simt=False):
-    """q,k,v: (B,T,H,D) logical bf16 views.  Returns o (B,T,H,D) contiguous bf16, lse (B,H,T) fp32 or None."""
+def attn_fwd_raw(q, k, v, cos, sin, meta, scale, need_lse=True, simt=False, q_offset=0):
+    """q: (B,T,H,D), k,v: (B,q_offset+T,H,D) logical bf16 views; the queries are key rows [q_offset, q_offset+T) and
+    the metadata is in key coordinates (a continuation chunk onto a KV cache; 0 = prefill).  cos/sin have T rows.
+    Returns o (B,T,H,D) contiguous bf16, lse (B,H,T) fp32 or None."""
     _require_cuda(q, k, v)
     B, T, H, D = q.shape
     o = torch.empty(B, T, H, D, dtype=torch.bfloat16, device=q.device)
     lse = torch.empty(B, H, T, dtype=torch.float32, device=q.device) if need_lse else None
     p = AttnParams()
-    _fill_params(p, q, k, v, o, lse, cos, sin, meta, scale)
+    _fill_params(p, q, k, v, o, lse, cos, sin, meta, scale, q_offset)
     fn = lib.aki_mma_attn_fwd_simt if simt else lib.aki_mma_attn_fwd
     check(fn(C.byref(p), _stream()), "aki_mma_attn_fwd" + ("_simt" if simt else ""))
     return o, lse
@@ -431,25 +457,33 @@ attn_packed_op.register_autograd(_packed_backward, setup_context=_packed_setup)
 # --------------------------------------------------------------------------------------------------
 @torch.library.custom_op("aki_mma::decode", mutates_args=())
 def decode_op(q: torch.Tensor, k_cache: torch.Tensor, v_cache: torch.Tensor, kv_len: torch.Tensor, max_kv_len: int,
-              scale: float, kv_start: _OT = None) -> torch.Tensor:
+              scale: float, kv_start: _OT = None, kv_valid_bits: _OT = None) -> torch.Tensor:
     """q (B,H,D) bf16 post-RoPE; caches (B,H,t_cap,D) bf16; kv_len (B,) int32; kv_start (B,) int32 or None (first
-    visible key: the leading pad rows of a left-padded prompt).  Returns (B,H,D) bf16."""
-    _require_cuda(q, k_cache, v_cache, kv_len, kv_start)
+    visible key: the leading pad rows of a left-padded prompt); kv_valid_bits (B, >= ceil(max_kv_len/32)) int32 or None
+    (keys whose bit is 0 are skipped: interior pad rows of a batched follow-up turn).  Returns (B,H,D) bf16."""
+    _require_cuda(q, k_cache, v_cache, kv_len, kv_start, kv_valid_bits)
     B, H, D = q.shape
     q = q.contiguous()
     out = torch.empty_like(q)
     nbytes = lib.aki_mma_decode_workspace_bytes(B, H, D, int(max_kv_len))
     ws = torch.empty(nbytes, dtype=torch.uint8, device=q.device)
     assert k_cache.stride(3) == 1 and k_cache.stride(2) == D and k_cache.stride() == v_cache.stride()
-    check(lib.aki_mma_decode(_ptr(q), _ptr(k_cache), _ptr(v_cache), k_cache.stride(0), k_cache.stride(1), _ptr(kv_len),
-                             _ptr(kv_start), int(max_kv_len), B, H, D, float(scale), _ptr(out), _ptr(ws), nbytes,
-                             _stream()),
-          "aki_mma_decode")
+    if kv_valid_bits is None:
+        check(lib.aki_mma_decode(_ptr(q), _ptr(k_cache), _ptr(v_cache), k_cache.stride(0), k_cache.stride(1),
+                                 _ptr(kv_len), _ptr(kv_start), int(max_kv_len), B, H, D, float(scale), _ptr(out), _ptr(ws),
+                                 nbytes, _stream()),
+              "aki_mma_decode")
+        return out
+    assert kv_valid_bits.dtype == torch.int32 and kv_valid_bits.is_contiguous() and kv_valid_bits.shape[0] == B
+    check(lib.aki_mma_decode_masked(_ptr(q), _ptr(k_cache), _ptr(v_cache), k_cache.stride(0), k_cache.stride(1),
+                                    _ptr(kv_len), _ptr(kv_start), _ptr(kv_valid_bits), kv_valid_bits.shape[1],
+                                    int(max_kv_len), B, H, D, float(scale), _ptr(out), _ptr(ws), nbytes, _stream()),
+          "aki_mma_decode_masked")
     return out
 
 
 @decode_op.register_fake
-def _(q, k_cache, v_cache, kv_len, max_kv_len, scale, kv_start=None):
+def _(q, k_cache, v_cache, kv_len, max_kv_len, scale, kv_start=None, kv_valid_bits=None):
     return torch.empty_like(q)
 
 

@@ -82,6 +82,13 @@ int aki_mma_segments(const int64_t* lang_x, const int64_t* attention_mask, int B
  *                                tiles before the diagonal plus everything from the diagonal on) */
 int aki_mma_tile_bounds(const int32_t* seq_len, const int32_t* row_lo, const int32_t* row_hi, int B, int T,
                         int t_cap, int32_t* q_tile_kv_end, uint32_t* kv_tile_q_mask, aki_stream_t stream);
+/* Same for the T query rows [q_offset, q_offset + T) of a continuation (see AkiMmaAttnParams.q_offset): query tile qt
+ * holds rows q_offset + [128 qt, 128 qt + 128) and q_tile_kv_end (B, ceil(T/128)) counts key tiles over
+ * [0, q_offset + T).  t_cap >= q_offset + T.  kv_tile_q_mask (backward only) must be NULL when q_offset != 0.
+ * aki_mma_tile_bounds(...) == aki_mma_tile_bounds_at(..., 0, ...). */
+int aki_mma_tile_bounds_at(const int32_t* seq_len, const int32_t* row_lo, const int32_t* row_hi, int B, int T,
+                           int q_offset, int t_cap, int32_t* q_tile_kv_end, uint32_t* kv_tile_q_mask,
+                           aki_stream_t stream);
 
 /* Forward work plan (ABI 2): the query rows of every sample cut into tiles of <= 128 rows that START at each image span
  * (so that a span of <= 128 vision tokens is ONE query tile instead of straddling two aligned ones -- with the
@@ -97,6 +104,14 @@ int aki_mma_tile_bounds(const int32_t* seq_len, const int32_t* row_lo, const int
 int aki_mma_fwd_plan(const int32_t* seq_len, const int32_t* row_lo, const int32_t* row_hi,
                      const uint32_t* kv_valid_bits, int B, int T, int meta_pitch, int bits_pitch, int max_pairs,
                      int flags, int32_t* plan, aki_stream_t stream);
+/* Plan of a continuation chunk (AkiMmaAttnParams.q_offset): cuts and pairs the T query rows [q_offset, q_offset + T)
+ * and counts key tiles over [0, q_offset + T); the tile starts it stores are chunk rows (0 = first query).  When the
+ * chunk starts off the 128-key grid, a first short tile realigns the following ones if that saves key-tile visits.
+ * meta_pitch >= q_offset + T, bits_pitch >= ceil((q_offset + T) / 32); row 0's first-bad key tile is absolute.
+ * aki_mma_fwd_plan(...) == aki_mma_fwd_plan_at(..., 0, ...). */
+int aki_mma_fwd_plan_at(const int32_t* seq_len, const int32_t* row_lo, const int32_t* row_hi,
+                        const uint32_t* kv_valid_bits, int B, int T, int q_offset, int meta_pitch, int bits_pitch,
+                        int max_pairs, int flags, int32_t* plan, aki_stream_t stream);
 
 /* Debug / parity helper: expand the compact description to the reference's (B,1,T,T) int64 0/1 tensor
  * (what _prepare_inputs_for_forward returns under "attention_mask", vlm.py:589-603). */
@@ -155,23 +170,25 @@ typedef struct AkiMmaTensor4 { /* logical (B, T, H, D) bf16 view, last dim conti
 } AkiMmaTensor4;
 
 typedef struct AkiMmaAttnParams {
-  int32_t B, H, T, D; /* queries == keys == T (prefill / training); D == 96 */
+  int32_t B, H, T, D; /* T queries against q_offset + T keys (q_offset = 0: prefill / training); D == 96 */
   float scale;        /* softmax scale, 1/sqrt(96) */
-  AkiMmaTensor4 q;    /* pre-RoPE if rope_cos != NULL, else used as is */
-  AkiMmaTensor4 k;    /* post-RoPE keys (cache layout or any strided view) */
-  AkiMmaTensor4 v;
+  AkiMmaTensor4 q;    /* (B,T,H,D); pre-RoPE if rope_cos != NULL, else used as is */
+  AkiMmaTensor4 k;    /* (B,q_offset+T,H,D) post-RoPE keys (cache layout or any strided view) */
+  AkiMmaTensor4 v;    /* (B,q_offset+T,H,D) */
   AkiMmaTensor4 o;    /* output, (B,T,H,D) view */
   float* lse;         /* (B,H,T) fp32 natural-log sum-exp of scaled scores; may be NULL (inference) */
-  const float* rope_cos; /* (B or 1, T, D/2) fp32 or NULL: rotate Q while loading it */
+  const float* rope_cos; /* (B or 1, T, D/2) fp32 or NULL: rotate Q while loading it (row r of the table = query r) */
   const float* rope_sin;
   int64_t rope_stride_b;
-  /* MMA description; all NULL => plain causal over T keys */
+  /* MMA description in KEY coordinates (row i of the metadata = absolute row i of the q_offset + T key sequence; query r
+   * is absolute row q_offset + r; rows below q_offset are never read); all NULL => plain causal over the keys.
+   * seq_len <= q_offset + T, meta_pitch >= q_offset + T, bits_pitch >= ceil((q_offset + T) / 32). */
   const int32_t* seq_len;          /* (B) */
   const int32_t* row_lo;           /* (B, meta_pitch) */
   const int32_t* row_hi;           /* (B, meta_pitch) */
   const uint32_t* kv_valid_bits;   /* (B, bits_pitch) */
   const uint32_t* kv_mutual_bits;  /* (B, bits_pitch) */
-  const int32_t* q_tile_kv_end;    /* (B, ceil(T/128)) */
+  const int32_t* q_tile_kv_end;    /* (B, ceil(T/128)): key tiles of each 128-row QUERY tile (aki_mma_tile_bounds_at) */
   const uint32_t* kv_tile_q_mask;  /* (B, ceil(T/128), ceil(ceil(T/128)/32)); backward only */
   int32_t meta_pitch, bits_pitch;
   /* ABI 2: forward work plan from aki_mma_fwd_plan ((B, 1 + plan_pairs) x 4 int32), or NULL: aligned 128-row query
@@ -179,7 +196,12 @@ typedef struct AkiMmaAttnParams {
    * against the predicate -- correct, slower). */
   const int32_t* fwd_plan;
   int32_t plan_pairs;
-  int32_t reserved0;
+  /* Continuation onto a KV cache (follow-up turn, chunked prefill): the T queries are rows [q_offset, q_offset + T) of
+   * the key sequence.  q, o, lse and the RoPE tables have T rows; k, v and the metadata above cover q_offset + T rows
+   * (a plan from aki_mma_fwd_plan_at, kv ends from aki_mma_tile_bounds_at with the same q_offset).  0 = prefill.
+   * q_offset < 0 or q_offset + T > INT32_MAX: AKI_ERR_BAD_SHAPE.  The backward refuses q_offset != 0
+   * (AKI_ERR_UNSUPPORTED): training never continues onto a cache. */
+  int32_t q_offset;
 } AkiMmaAttnParams;
 
 int aki_mma_attn_fwd(const AkiMmaAttnParams* p, aki_stream_t stream);
@@ -209,6 +231,13 @@ size_t aki_mma_decode_workspace_bytes(int B, int H, int D, int max_kv_len);
 int aki_mma_decode(const void* q, const void* k_cache, const void* v_cache, int64_t cache_stride_b,
                    int64_t cache_stride_h, const int32_t* kv_len, const int32_t* kv_start, int max_kv_len, int B, int H,
                    int D, float scale, void* out, void* workspace, size_t workspace_bytes, aki_stream_t stream);
+/* Same, skipping every key whose bit in kv_valid_bits (B, bits_pitch) uint32 is 0 (bit j of word j/32 = key j): a
+ * batched follow-up turn appends left-padded prompts, so the cache holds invalid rows in its interior, which kv_start
+ * cannot describe.  bits_pitch * 32 >= max_kv_len.  kv_valid_bits = NULL: aki_mma_decode. */
+int aki_mma_decode_masked(const void* q, const void* k_cache, const void* v_cache, int64_t cache_stride_b,
+                          int64_t cache_stride_h, const int32_t* kv_len, const int32_t* kv_start,
+                          const uint32_t* kv_valid_bits, int bits_pitch, int max_kv_len, int B, int H, int D, float scale,
+                          void* out, void* workspace, size_t workspace_bytes, aki_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------------------
  * (6) Decode-sized linear layers around the attention op (SURVEY 8 f-1, ABI 2) -- for B <= 8 tokens (one per sequence of
@@ -285,7 +314,8 @@ unsigned long long aki_mma_launch_count(void);
 
 /* ------------------------------------------------------------------------------------------------------
  * Verification kernels (tests only): the same maths as (4) written as plain SIMT CUDA with no tensor cores,
- * used to cross-check the tcgen05 kernels on-device at sizes the CPU oracle cannot reach. */
+ * used to cross-check the tcgen05 kernels on-device at sizes the CPU oracle cannot reach.  The forward honours
+ * q_offset like aki_mma_attn_fwd; the backward refuses it. */
 int aki_mma_attn_fwd_simt(const AkiMmaAttnParams* p, aki_stream_t stream);
 int aki_mma_attn_bwd_simt(const AkiMmaAttnBwdParams* p, aki_stream_t stream);
 
