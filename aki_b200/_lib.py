@@ -89,6 +89,9 @@ _SIGNATURES = {
                                         C.c_void_p, C.c_size_t, C.c_void_p]),
     "aki_mma_skinny_linear": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_float, C.c_void_p, C.c_int64,
                                         C.c_void_p, C.c_int64, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]),
+    "aki_mma_batch_linear": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_float, C.c_void_p, C.c_int64,
+                                       C.c_void_p, C.c_int64, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]),
+    "aki_mma_batch_linear_split": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int]),
     "aki_mma_add_rmsnorm": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p, C.c_float, C.c_void_p,
                                       C.c_int64, C.c_void_p, C.c_int64, C.c_int, C.c_int, C.c_void_p]),
     "aki_mma_swiglu": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_int, C.c_int, C.c_void_p]),

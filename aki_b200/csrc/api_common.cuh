@@ -47,8 +47,32 @@ inline void launch_pdl(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t sme
   cfg.numAttrs = pdl_enabled() ? 1 : 0;
   cudaLaunchKernelEx(&cfg, kern, static_cast<KArgs>(args)...);
 }
+// Same, with thread-block clusters of `cluster_x` CTAs along grid x.
+template <typename... KArgs, typename... Args>
+inline void launch_pdl_cluster(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st,
+                               unsigned cluster_x, Args&&... args) {
+  cudaLaunchConfig_t cfg = {};
+  cfg.gridDim = grid;
+  cfg.blockDim = block;
+  cfg.dynamicSmemBytes = smem;
+  cfg.stream = st;
+  cudaLaunchAttribute attr[2];
+  attr[0].id = cudaLaunchAttributeClusterDimension;
+  attr[0].val.clusterDim.x = cluster_x;
+  attr[0].val.clusterDim.y = 1;
+  attr[0].val.clusterDim.z = 1;
+  attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  attr[1].val.programmaticStreamSerializationAllowed = 1;
+  cfg.attrs = attr;
+  cfg.numAttrs = pdl_enabled() ? 2 : 1;
+  cudaLaunchKernelEx(&cfg, kern, static_cast<KArgs>(args)...);
+}
 
 inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
+
+// (cols, rows) bf16 matrix with a row stride in elements -> TMA map of [32 x box_rows] SWIZZLE_64B boxes, the K-major
+// UMMA operand layout (sm100_ptx.cuh sw64_offset); rows past the end load as zeros.  attn_fwd_sm100.cu.
+int make_bf16_map_2d(CUtensorMap* m, const void* base, int cols, int rows, int64_t row_stride, int box_rows);
 
 #define AKI_REQUIRE(cond, code) \
   do {                          \

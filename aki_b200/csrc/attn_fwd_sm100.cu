@@ -726,6 +726,22 @@ int make_tile_map(CUtensorMap* m, const AkiMmaTensor4& t, int B, int H, int T, i
   return AKI_OK;
 }
 
+// (cols, rows) bf16 matrix, row stride in elements -> tensor map with [32 x box_rows] SWIZZLE_64B boxes (rows past the
+// end read as zeros)
+int make_bf16_map_2d(CUtensorMap* m, const void* base, int cols, int rows, int64_t row_stride, int box_rows) {
+  EncodeTiledFn enc = get_encode_fn();
+  if (!enc) { set_last_cuda_error("cuTensorMapEncodeTiled entry point not found"); return AKI_ERR_CUDA; }
+  cuuint64_t dims[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
+  cuuint64_t strides[1] = {(cuuint64_t)row_stride * 2};
+  cuuint32_t box[2] = {32, (cuuint32_t)box_rows};
+  cuuint32_t es[2] = {1, 1};
+  CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(base), dims, strides, box, es,
+                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  if (r != CUDA_SUCCESS) { set_last_cuda_error("cuTensorMapEncodeTiled(2d) failed"); return AKI_ERR_CUDA; }
+  return AKI_OK;
+}
+
 // dQ accumulator (B,H,T,96) fp32 contiguous -> [32 x 128 x 1 x 1] fp32 SWIZZLE_128B boxes for TMA reductions
 int make_dq_accum_map(CUtensorMap* m, float* dq_accum, int B, int H, int T) {
   EncodeTiledFn enc = get_encode_fn();

@@ -93,6 +93,39 @@ __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
 #endif
 }
 
+// ---------------------------------------------------------------------------------------------- cluster (DSMEM)
+// Every CTA of the cluster, all threads: orders the shared-memory state (barrier inits) of each CTA before any access
+// from another CTA of the cluster.
+__device__ __forceinline__ void cluster_sync() {
+  asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
+}
+// Address of the same shared-memory location in CTA `rank` of the cluster.
+__device__ __forceinline__ uint32_t mapa_shared(uint32_t addr, uint32_t rank) {
+  uint32_t r;
+  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(addr), "r"(rank));
+  return r;
+}
+__device__ __forceinline__ void st_cluster_f32(uint32_t addr, float v) {
+  asm volatile("st.shared::cluster.f32 [%0], %1;" ::"r"(addr), "f"(v) : "memory");
+}
+// Arrive on an mbarrier of any CTA of the cluster, releasing this thread's earlier writes at cluster scope.
+__device__ __forceinline__ void mbar_arrive_cluster(uint32_t bar_cluster_addr) {
+  asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(bar_cluster_addr) : "memory");
+}
+// mbar_wait with cluster-scope acquire: the phase was completed by arrivals of other CTAs (mbar_arrive_cluster).
+__device__ __forceinline__ void mbar_wait_cluster(uint32_t bar, uint32_t parity) {
+  uint32_t ok = 0;
+  while (!ok) {
+    asm volatile(
+        "{\n\t.reg .pred P;\n\t"
+        "mbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 P, [%1], %2, %3;\n\t"
+        "selp.b32 %0, 1, 0, P;\n\t}\n"
+        : "=r"(ok)
+        : "r"(bar), "r"(parity), "r"(AKI_MBAR_SUSPEND_NS)
+        : "memory");
+  }
+}
+
 // ---------------------------------------------------------------------------------------------- work queue
 // Cluster launch control: ask the hardware queue for the next not-yet-started CTA of this grid.
 __device__ __forceinline__ void clc_try_cancel(uint32_t resp_smem, uint32_t bar) {
@@ -135,6 +168,12 @@ __device__ __forceinline__ void tma_load_4d(uint32_t dst, const CUtensorMap* m, 
   asm volatile(
       "cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];"
       ::"r"(dst), "l"(reinterpret_cast<uint64_t>(m)), "r"(bar), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
+      : "memory");
+}
+__device__ __forceinline__ void tma_load_2d(uint32_t dst, const CUtensorMap* m, uint32_t bar, int c0, int c1) {
+  asm volatile(
+      "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
+      ::"r"(dst), "l"(reinterpret_cast<uint64_t>(m)), "r"(bar), "r"(c0), "r"(c1)
       : "memory");
 }
 __device__ __forceinline__ void tma_store_4d(const CUtensorMap* m, uint32_t src, int c0, int c1, int c2, int c3) {

@@ -106,7 +106,7 @@ class AkiPhi3Runner(nn.Module):
     # ---- fused decode layers ("next" row f-1 of SURVEY 8): 7 launches per layer instead of ~15 --------------------------
     @torch.no_grad()
     def _fused_layers(self, h: torch.Tensor, cos, sin, cache: AkiKVCache, past: Optional[int]):
-        """One decode step through all decoder layers for h (B<=8, 3072): RMSNorm->qkv_proj, RoPE + KV write, decode
+        """One decode step through all decoder layers for h (B<=64, 3072): RMSNorm->qkv_proj, RoPE + KV write, decode
         attention, o_proj + residual, RMSNorm->gate_up_proj->SiLU gate, down_proj + residual -- each GEMM one
         weight-streaming kernel (ops.skinny_linear) with the norm / activation / residual fused in.  past=None: the write
         row and key count come from device memory (CUDA-graph replay).  Returns the last-layer hidden state (B,3072)."""
@@ -136,7 +136,7 @@ class AkiPhi3Runner(nn.Module):
         past = cache.get_seq_length()
         cache._check(past + 1)
         B = token_ids.shape[0]
-        if B > 8:
+        if B > 64:
             return self.decode_step(token_ids, cache)
         h = self.lm.model.embed_tokens(token_ids).view(B, -1)
         pos = torch.full((1, 1), past, device=h.device, dtype=torch.long)
@@ -167,7 +167,7 @@ class AkiPhi3Runner(nn.Module):
 
     @torch.no_grad()
     def decode_step_graphed(self, token_ids: torch.Tensor, cache: AkiKVCache, fused: bool = True) -> torch.Tensor:
-        """Greedy decode step replayed from a CUDA graph: returns the next token ids (B,1).  fused (default, B <= 8): the
+        """Greedy decode step replayed from a CUDA graph: returns the next token ids (B,1).  fused (default, B <= 64): the
         layers run through the weight-streaming kernels of _fused_layers.  A graph is captured on first
         use for this cache and for each longrope factor set; the write row, the key count and the position id live in
         device memory (cache.past_dev), so replays need no host-side arguments.  The factor set follows the running
@@ -175,7 +175,7 @@ class AkiPhi3Runner(nn.Module):
         while past + 1 <= original_max, long factors afterwards -- the step switches graphs when the boundary is crossed."""
         past = cache.get_seq_length()
         cache._check(past + 1)                                       # BEFORE anything is enqueued: the row must exist
-        fused = bool(fused) and token_ids.shape[0] <= 8
+        fused = bool(fused) and token_ids.shape[0] <= 64
         g = getattr(self, "_g", None)
         if g is None or g["cache"] is not cache or g["fused"] != fused:
             B = token_ids.shape[0]

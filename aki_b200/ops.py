@@ -492,20 +492,24 @@ def _(q, k_cache, v_cache, kv_len, max_kv_len, scale, kv_start=None, kv_valid_bi
 # --------------------------------------------------------------------------------------------------
 def skinny_linear(x: torch.Tensor, weight: torch.Tensor, rms_weight: _OT = None, rms_eps: float = 1e-5,
                   residual: _OT = None, swiglu: bool = False, out: _OT = None) -> torch.Tensor:
-    """y = epilogue(rmsnorm?(x) @ weight.T) for x (B<=8, K) bf16, weight (N or 2N, K) bf16 row-major:
+    """y = epilogue(rmsnorm?(x) @ weight.T) for x (B<=64, K) bf16, weight (N or 2N, K) bf16 row-major:
     residual -> y = residual + (.), swiglu -> y = up * silu(gate) (gate_up_proj layout).  One weight-streaming kernel
-    instead of Phi3RMSNorm + nn.Linear + activation / residual add (modeling_phi3.py:49-64, 295-335)."""
+    instead of Phi3RMSNorm + nn.Linear + activation / residual add (modeling_phi3.py:49-64, 295-335):
+    aki_mma_skinny_linear for B <= 8, aki_mma_batch_linear (tcgen05) for 9 <= B <= 64."""
     _require_cuda(x, weight, rms_weight, residual)
     assert x.dim() == 2 and x.dtype == torch.bfloat16 and weight.dtype == torch.bfloat16 and x.stride(1) == 1
     assert weight.is_contiguous() and weight.shape[1] == x.shape[1] and not (swiglu and residual is not None)
     B, K = x.shape
+    if B > 64:
+        raise ValueError(f"skinny_linear takes at most 64 tokens, got {B}")
     N = weight.shape[0] // (2 if swiglu else 1)
     if out is None:
         out = torch.empty(B, N, dtype=torch.bfloat16, device=x.device)
     mode = 2 if swiglu else (1 if residual is not None else 0)
-    check(lib.aki_mma_skinny_linear(_ptr(x), x.stride(0), _ptr(weight), _ptr(rms_weight), float(rms_eps), _ptr(residual),
-                                    residual.stride(0) if residual is not None else 0, _ptr(out), out.stride(0), B, N, K,
-                                    mode, _stream()), "aki_mma_skinny_linear")
+    fn = lib.aki_mma_skinny_linear if B <= 8 else lib.aki_mma_batch_linear
+    check(fn(_ptr(x), x.stride(0), _ptr(weight), _ptr(rms_weight), float(rms_eps), _ptr(residual),
+             residual.stride(0) if residual is not None else 0, _ptr(out), out.stride(0), B, N, K, mode, _stream()),
+          fn.__name__)
     return out
 
 

@@ -251,6 +251,17 @@ int aki_mma_decode_masked(const void* q, const void* k_cache, const void* v_cach
 int aki_mma_skinny_linear(const void* x, int64_t x_stride, const void* w, const void* rms_weight, float rms_eps,
                           const void* residual, int64_t residual_stride, void* y, int64_t y_stride, int B, int N, int K,
                           int mode, aki_stream_t stream);
+/* Same contract, argument for argument, for 1 <= B <= 64 tokens (a batched decode step), on tcgen05 tensor cores: the
+ * weights stream through a TMA ring, the K range of each 128-row tile is split over a cluster of CTAs and reduced in a
+ * fixed order through distributed shared memory (deterministic, no workspace).  N % 16 == 0; K % 64 == 0; x_stride
+ * % 8 == 0 and x_stride >= K when B > 1; strides in elements.  Same status codes as aki_mma_skinny_linear.  Row b of the
+ * output depends on B only through roundup(B, 16).  HBM-bound: N*K*2 bytes per call (x2 in mode 2).
+ * aki_mma_batch_linear_split: the number of CTAs (1 - 8) a call with these arguments splits K over, or a negative
+ * status; needs a current device. */
+int aki_mma_batch_linear(const void* x, int64_t x_stride, const void* w, const void* rms_weight, float rms_eps,
+                         const void* residual, int64_t residual_stride, void* y, int64_t y_stride, int B, int N, int K,
+                         int mode, aki_stream_t stream);
+int aki_mma_batch_linear_split(int B, int N, int K, int mode);
 
 /* ------------------------------------------------------------------------------------------------------
  * (7) Element-wise work of the decoder layer at PREFILL size (SURVEY 8 f-1, ABI 2) -- one pass over HBM each, replacing
