@@ -49,6 +49,11 @@ class AttnBwdParams(C.Structure):
     ]
 
 
+class AdamWTensor(C.Structure):
+    _fields_ = [("param", C.c_void_p), ("grad", C.c_void_p), ("exp_avg", C.c_void_p), ("exp_avg_sq", C.c_void_p),
+                ("param_bf16", C.c_void_p), ("numel", C.c_int64)]
+
+
 _SIGNATURES = {
     "aki_mma_abi_version": (C.c_int, []),
     "aki_mma_strerror": (C.c_char_p, [C.c_int]),
@@ -106,6 +111,10 @@ _SIGNATURES = {
     "aki_mma_rmsnorm_amp_bwd": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                           C.c_void_p, C.c_int, C.c_int, C.c_void_p]),
     "aki_mma_swiglu_bwd": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p]),
+    "aki_mma_grad_sq_norm_workspace_bytes": (C.c_size_t, [C.c_void_p, C.c_int]),
+    "aki_mma_grad_sq_norm": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p]),
+    "aki_mma_adamw_step": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_float, C.c_float, C.c_float, C.c_float, C.c_float,
+                                     C.c_float, C.c_int64, C.c_void_p]),
     "aki_mma_set_timing_events": (C.c_int, [C.c_void_p, C.c_void_p]),
     "aki_mma_launch_count": (C.c_ulonglong, []),
     "aki_mma_attn_fwd_simt": (C.c_int, [C.POINTER(AttnParams), C.c_void_p]),

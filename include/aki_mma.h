@@ -312,6 +312,41 @@ int aki_mma_rmsnorm_amp_bwd(const void* dx, const float* dh_out, const float* h,
                             float* dh, float* dw_partial, int M, int K, aki_stream_t stream);
 int aki_mma_swiglu_bwd(const void* d_out, const void* gate_up, void* d_gate_up, int M, int N, aki_stream_t stream);
 
+/* ------------------------------------------------------------------------------------------------------
+ * (10) Optimizer step of the SFT loop -- replaces torch.nn.utils.clip_grad_norm_ + torch.optim.AdamW.step of the
+ *      reference's training step (train_utils.py:143-158) and, through the bf16 parameter copy it writes, autocast's
+ *      fp32 -> bf16 weight cast in every forward (configs/sft.yaml:55 amp_bf16).  Two HBM-bound passes over a list of
+ *      fp32 tensors, given as a HOST array of entries (copied into the kernels' parameter space: no device table; longer
+ *      lists than one launch takes are split into several launches by the library).  Every pointer is 16-byte aligned.
+ *   aki_mma_grad_sq_norm: *sq_norm (device, 1 float) = sum of grad^2 over every entry.  Reads `grad` and `numel` only.
+ *     Fixed-order reduction (fp32 partials of 16384 elements, added in fp64 in chunk order): the same inputs give the
+ *     same bits on every run.  workspace: aki_mma_grad_sq_norm_workspace_bytes(t, n) bytes (0 for an invalid list).
+ *   aki_mma_adamw_step: per element, with c = min(1, max_norm / (sqrt(*sq_norm) + 1e-6)) (c = 1 when sq_norm is NULL;
+ *     a NaN norm gives c = NaN, an infinite one c = 0, as clip_grad_norm_ does):
+ *       g = grad * c;  param -= lr * weight_decay * param;  exp_avg = lerp(exp_avg, g, 1 - beta1);
+ *       exp_avg_sq = lerp(exp_avg_sq, g^2, 1 - beta2);
+ *       param -= lr / (1 - beta1^step) * exp_avg / (sqrt(exp_avg_sq) / sqrt(1 - beta2^step) + eps)
+ *     in the fp32 operations of torch.optim.AdamW(fused=True); then param_bf16 (when non-NULL) = bf16(param), rounded to
+ *     nearest even like param.to(torch.bfloat16).  `grad` is NOT rescaled in place (clip_grad_norm_ rescales it).
+ *     step >= 1 is the step count after this update; 0 <= beta < 1, lr, eps, weight_decay finite and >= 0, max_norm
+ *     finite and > 0 when sq_norm is given; otherwise AKI_ERR_BAD_SHAPE.
+ *   All status codes are returned before any launch: AKI_ERR_NULL (t, a required pointer of a non-empty entry,
+ *   workspace, sq_norm), AKI_ERR_BAD_SHAPE (n <= 0, numel < 0, hyperparameters, workspace too small), AKI_ERR_MISALIGNED. */
+typedef struct AkiAdamWTensor {
+  float* param;
+  const float* grad;
+  float* exp_avg;
+  float* exp_avg_sq;
+  void* param_bf16;   /* bf16 copy written after the update, or NULL */
+  int64_t numel;
+} AkiAdamWTensor;
+
+size_t aki_mma_grad_sq_norm_workspace_bytes(const AkiAdamWTensor* t, int n);
+int aki_mma_grad_sq_norm(const AkiAdamWTensor* t, int n, void* workspace, size_t workspace_bytes, float* sq_norm,
+                         aki_stream_t stream);
+int aki_mma_adamw_step(const AkiAdamWTensor* t, int n, const float* sq_norm, float max_norm, float lr, float beta1,
+                       float beta2, float eps, float weight_decay, int64_t step, aki_stream_t stream);
+
 /* Measurement hook (bench.py roofline): the NEXT aki_mma_attn_fwd / aki_mma_attn_bwd call of this host thread
  * records `ev_begin` right before and `ev_end` right after its tcgen05 attention kernel on the call's stream (the
  * preprocess / memset / finalize launches of the backward stay outside), then the hook clears itself.

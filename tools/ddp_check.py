@@ -1,5 +1,6 @@
 """DDP check for the SFT step (BASELINE config 4, SURVEY 8e): gradients of a 2-rank DDP step (per-rank batch 2) must
-equal the gradients of the same 4 samples run as one batch on a single GPU, and batch-sharded prefill must equal the
+equal the gradients of the same 4 samples run as one batch on a single GPU; a DDP step with AkiAdamW + use_bf16_weights
+(bucket views, static graph) must update the parameters like that single-GPU step; batch-sharded prefill must equal the
 unsharded prefill.  Launch:  python -m torch.distributed.run --nnodes=1 --nproc-per-node 2 --master-addr 127.0.0.1
 --master-port 29511 tools/ddp_check.py      (gpurun --gpus 2)"""
 import os
@@ -65,6 +66,30 @@ def main():
     t = torch.tensor([worst], device=dev)
     dist.all_reduce(t, op=dist.ReduceOp.MAX)
 
+    # AkiAdamW + the bf16 weight copies under DDP: one clipped step on the shards moves the parameters like the same step
+    # on the full batch on one GPU (relative to the size of the update)
+    def fused_step(ddp):
+        m2 = AkiPhi3SFT(cfg, device=dev, seed=0)
+        p0 = [p.detach().clone() for p in m2.parameters()]
+        opt = aki_b200.AkiAdamW(m2.parameters(), lr=1e-4, weight_decay=1e-4, max_grad_norm=1.0)
+        aki_b200.use_bf16_weights(m2, opt)
+        me.lang_model = m2.lm
+        if ddp:
+            n2 = DDP(m2, device_ids=[local], gradient_as_bucket_view=True, static_graph=True)
+            l2, _ = loss_of(n2, si, sa, sl, sv)
+            (l2 * (n_tok * world / n_tok_full)).backward()
+        else:
+            l2, _ = loss_of(m2, ids, amt, lab, vis)
+            l2.backward()
+        opt.step()
+        return [p.detach() - q for p, q in zip(m2.parameters(), p0)]
+
+    d_ref, d_ddp = fused_step(False), fused_step(True)
+    num = sum(float((a - b).double().pow(2).sum()) for a, b in zip(d_ddp, d_ref)) ** 0.5
+    den = sum(float(b.double().pow(2).sum()) for b in d_ref) ** 0.5
+    t_opt = torch.tensor([num / (den + 1e-30)], device=dev)
+    dist.all_reduce(t_opt, op=dist.ReduceOp.MAX)
+
     # batch-sharded prefill == unsharded prefill (no collective on the data path; results gathered afterwards)
     runner = AkiPhi3Runner(cfg, device=dev, seed=0)
     me.lang_model = runner.lm
@@ -76,8 +101,9 @@ def main():
     gathered = gather_batch(part, B)
     e_pf = float((gathered.float().cpu() - full.float().cpu()).abs().max())
     if rank == 0:
-        ok = float(t[0]) < 3e-2 and e_pf < 5e-2
+        ok = float(t[0]) < 3e-2 and float(t_opt[0]) < 3e-2 and e_pf < 5e-2
         print(f"ddp_check world={world}: max relative grad error vs single-GPU full batch = {float(t[0]):.3e}; "
+              f"AkiAdamW + bf16 weights step, |update - single-GPU update| / |update| = {float(t_opt[0]):.3e}; "
               f"sharded-vs-unsharded prefill logits max abs diff = {e_pf:.3e}  ->  {'PASS' if ok else 'FAIL'}")
     dist.destroy_process_group()
 
