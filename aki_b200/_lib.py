@@ -130,14 +130,11 @@ def _load():
             f"{LIB_PATH} is missing: the CUDA library is the product and there is no fallback. Build it with "
             f"`python -c 'import __graft_entry__ as g; g.build()'` or `make -C aki_b200/csrc`.")
     lib = C.CDLL(LIB_PATH)
-    compat = bool(os.environ.get("AKI_MMA_LIB_COMPAT"))   # tools only: time the FORWARD of an ABI-1 build (same-box A/B)
     for name, (res, args) in _SIGNATURES.items():
-        if compat and not hasattr(lib, name):
-            continue
         fn = getattr(lib, name)          # AttributeError if the ABI is incomplete
         fn.restype = res
         fn.argtypes = args
-    if lib.aki_mma_abi_version() != ABI_VERSION and not compat:
+    if lib.aki_mma_abi_version() != ABI_VERSION:
         raise ImportError(f"{LIB_PATH}: ABI version {lib.aki_mma_abi_version()} != {ABI_VERSION}; rebuild")
     return lib
 

@@ -1,7 +1,6 @@
 // Status strings / diagnostics of the C ABI (include/aki_mma.h).
 #include <string.h>
 #include <atomic>
-#include <stdlib.h>
 #include "api_common.cuh"
 
 namespace aki {
@@ -12,10 +11,6 @@ void set_last_cuda_error(const char* msg) {
 }
 static std::atomic<unsigned long long> g_launches{0};
 void count_launch() { g_launches.fetch_add(1, std::memory_order_relaxed); }
-bool pdl_enabled() {
-  static const bool on = []() { const char* e = getenv("AKI_MMA_PDL"); return !(e && e[0] == '0'); }();
-  return on;
-}
 static thread_local cudaEvent_t g_ev_begin = nullptr, g_ev_end = nullptr;
 void timing_hook_begin(cudaStream_t st) {
   if (g_ev_begin) cudaEventRecord(g_ev_begin, st);

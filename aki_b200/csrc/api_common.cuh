@@ -29,8 +29,6 @@ inline int check_launch() {
 // griddepcontrol.launch_dependents, and run up to their own griddepcontrol.wait -- which returns once the previous
 // kernel has completed and its writes are visible.  Kernels launched this way execute pdl_prologue() before they touch
 // memory another kernel may have written (weights, which no kernel writes, may be requested earlier).
-// AKI_MMA_PDL=0: plain stream order.
-bool pdl_enabled();
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 __device__ __forceinline__ void pdl_trigger() { asm volatile("griddepcontrol.launch_dependents;"); }
 template <typename... KArgs, typename... Args>
@@ -44,7 +42,7 @@ inline void launch_pdl(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t sme
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = pdl_enabled() ? 1 : 0;
+  cfg.numAttrs = 1;
   cudaLaunchKernelEx(&cfg, kern, static_cast<KArgs>(args)...);
 }
 // Same, with thread-block clusters of `cluster_x` CTAs along grid x.
@@ -64,7 +62,7 @@ inline void launch_pdl_cluster(void (*kern)(KArgs...), dim3 grid, dim3 block, si
   attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[1].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = pdl_enabled() ? 2 : 1;
+  cfg.numAttrs = 2;
   cudaLaunchKernelEx(&cfg, kern, static_cast<KArgs>(args)...);
 }
 

@@ -71,9 +71,7 @@ constexpr int SMEM_ZERO = SMEM_ONES_D + 128;                // one all-zero core
 constexpr int SLOTS = 2;                      // item ring: the current item and the next one
 constexpr int SMEM_QLIST = SMEM_ZERO + 128;                 // SLOTS x uint16[MAX_TILES]
 constexpr int SMEM_TOTAL = SMEM_QLIST + SLOTS * MAX_TILES * 2;
-#ifndef AKI_BWD_SLICES_PER_GROUP
-#define AKI_BWD_SLICES_PER_GROUP 8
-#endif
+constexpr int SLICES_PER_GROUP = 8;           // (batch, head) slices per item group (header comment)
 constexpr int SMEM_ALLOC = SMEM_TOTAL + 1024;
 static_assert(SMEM_ALLOC + 256 <= 232448, "shared memory budget");
 constexpr uint32_t TM_S = 0, TM_DP = 128, TM_DV = 256, TM_DK = 352, TM_P = 448;
@@ -87,16 +85,16 @@ struct BwdKernelParams {
   int64_t rope_stride_b;
   MaskMeta mm;
   int B, H, T, n_t, n_words;
-  int group, n_items, use_clc;   // items: ((g * n_t + kt) * group + slice)
+  int group;             // items: ((g * n_t + kt) * group + slice); the grid has one CTA per item
   float scale_log2, scale;
-  unsigned long long* trace;  // debug build (make TRACE=1, tools/bwd_trace.py): clock64 stamps of one CTA
+  unsigned long long* trace;  // trace build (-DAKI_FWD_TRACE, tools/bwd_trace.py): clock64 stamps of one CTA
   int trace_cta;
 };
 
-// -DKO_x (tools/build_bwd_ko.sh) are timing-only knockout builds: each removes one component -- an MMA group (KO_S KO_DP
-// KO_DV KO_DQ KO_DK), the ex2 (KO_EXP), the dS compute + store + proxy fence (KO_DS; KO_FENCE only the fence), the dQ
-// drain (KO_DRAIN; KO_RED only its reductions), the Q/dO loads after the first ring fill (KO_TMA).  Results are wrong by
-// construction; the shipped build defines none of them.
+// -DKO_x (tools/build_variant.sh ko_x -DKO_x) are timing-only knockout builds: each removes one component -- an MMA group
+// (KO_S KO_DP KO_DV KO_DQ KO_DK), the ex2 (KO_EXP), the dS compute + store + proxy fence (KO_DS; KO_FENCE only the fence),
+// the dQ drain (KO_DRAIN; KO_RED only its reductions), the Q/dO loads after the first ring fill (KO_TMA).  Results are
+// wrong by construction; the shipped build defines none of them.
 #ifdef AKI_FWD_TRACE
 #define TRB(slot, j, k) do { if (tracing && (j) < 64) P.trace[((slot) * 64 + (j)) * 8 + (k)] = clock64(); } while (0)
 #else
@@ -494,22 +492,17 @@ attn_bwd_sm100_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_co
         }
         ++n_pub;
       }
-      // next item: the hardware queue, or a fixed stride (A/B builds)
+      // next item from the hardware queue
       int more = 0;
       long long next = 0;
       if (lane == 0) {
-        if (!P.use_clc) {
-          next = id + gridDim.x;
-          more = next < P.n_items;
-        } else {
-          mbar_arrive_expect_tx(BAR(CLC_BAR), 16);
-          clc_try_cancel(smem_u32(&clc_resp), BAR(CLC_BAR));
-          mbar_wait(BAR(CLC_BAR), n_clc & 1);
-          uint32_t x;
-          more = clc_query(smem_u32(&clc_resp), x) ? 1 : 0;
-          next = x;
-          fence_proxy_async_smem();     // the response buffer is rewritten by the next (async-proxy) query
-        }
+        mbar_arrive_expect_tx(BAR(CLC_BAR), 16);
+        clc_try_cancel(smem_u32(&clc_resp), BAR(CLC_BAR));
+        mbar_wait(BAR(CLC_BAR), n_clc & 1);
+        uint32_t x;
+        more = clc_query(smem_u32(&clc_resp), x) ? 1 : 0;
+        next = x;
+        fence_proxy_async_smem();     // the response buffer is rewritten by the next (async-proxy) query
       }
       ++n_clc;
       more = __shfl_sync(0xffffffffu, more, 0);
@@ -805,24 +798,21 @@ attn_bwd_sm100_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_co
   if (warp == 2) tmem_dealloc<512>(tmem);
 }
 
-// Per-device one-time setup (kernel attribute, SM count): the library may drive several GPUs from one process.
+// Per-device one-time setup (kernel attribute): the library may drive several GPUs from one process.
 struct BwdDeviceState {
   std::once_flag once;
-  int sm_count = 0;
   cudaError_t err = cudaSuccess;
 };
 static BwdDeviceState g_bwd_dev[64];
 
-static int bwd_device_setup(int* sm_count) {
+static int bwd_device_setup() {
   int dev = 0;
   if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) { set_last_cuda_error("cudaGetDevice failed"); return AKI_ERR_CUDA; }
   BwdDeviceState& s = g_bwd_dev[dev];
   std::call_once(s.once, [&]() {
     s.err = cudaFuncSetAttribute(attn_bwd_sm100_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, bwd::SMEM_ALLOC);
-    if (s.err == cudaSuccess) s.err = cudaDeviceGetAttribute(&s.sm_count, cudaDevAttrMultiProcessorCount, dev);
   });
   if (s.err != cudaSuccess) { set_last_cuda_error(cudaGetErrorString(s.err)); return AKI_ERR_CUDA; }
-  *sm_count = s.sm_count;
   return AKI_OK;
 }
 
@@ -879,19 +869,13 @@ extern "C" int aki_mma_attn_bwd(const AkiMmaAttnBwdParams* p, aki_stream_t strea
   }
 #endif
   const long long slices = (long long)f.B * f.H;
-  kp.group = (int)(slices < AKI_BWD_SLICES_PER_GROUP ? slices : AKI_BWD_SLICES_PER_GROUP);
+  kp.group = (int)(slices < bwd::SLICES_PER_GROUP ? slices : bwd::SLICES_PER_GROUP);
   const long long n_groups = (slices + kp.group - 1) / kp.group;
   const long long n_items = n_groups * kp.n_t * kp.group;
   AKI_REQUIRE(n_items > 0 && n_items < (1ll << 31), AKI_ERR_BAD_SHAPE);
-  kp.n_items = (int)n_items;
-  int sm_count = 0;
-  if ((rc = bwd_device_setup(&sm_count))) return rc;
-  // AKI_MMA_BWD_SCHED=static: persistent CTAs walk the items with a fixed stride instead of the hardware queue (A/B only)
-  static const bool use_static = []() { const char* e = getenv("AKI_MMA_BWD_SCHED"); return e && e[0] == 's'; }();
-  kp.use_clc = use_static ? 0 : 1;
-  const long long grid = kp.use_clc ? n_items : (n_items < sm_count ? n_items : sm_count);
+  if ((rc = bwd_device_setup())) return rc;
   timing_hook_begin(st);
-  attn_bwd_sm100_kernel<<<(unsigned)grid, bwd::THREADS, bwd::SMEM_ALLOC, st>>>(mq, mk, mv, mdo, mdq, mqa, kp);
+  attn_bwd_sm100_kernel<<<(unsigned)n_items, bwd::THREADS, bwd::SMEM_ALLOC, st>>>(mq, mk, mv, mdo, mdq, mqa, kp);
   timing_hook_end(st);
 #ifdef AKI_FWD_TRACE
   if (trace_env) {

@@ -41,13 +41,6 @@
 #include "attn_aux.cuh"
 #include "sm100_ptx.cuh"
 
-#ifndef AKI_FWD_POLY
-#define AKI_FWD_POLY 0         // of every 4 score pairs, how many take the polynomial exp2 (FMA pipe) instead of MUFU.EX2
-#endif                         // (same box, causal / 4 images: 0 -> 0.88 / 1.06 ms, 1 -> 0.87-0.99 / 1.04-1.19 depending on
-                               // code placement, 2 -> 0.96 / 1.14, 3 -> 1.03 / 1.24: the softmax warps are bound by their
-                               // own instruction stream, not by the MUFU pipe -- tools/mufu_bench.cu)
-
-
 namespace aki {
 
 namespace fwd {
@@ -63,10 +56,7 @@ constexpr int SMEM_ALLOC = SMEM_TOTAL + 1024;              // slack for 1024-byt
 constexpr uint32_t TM_S = 0, TM_O = 256, TM_P = 448;       // S: 128 t; O: 96 t; P: 32 t
 constexpr int REGS_CTRL = 56, REGS_SOFTMAX = 192, REGS_EPI = 72;   // 128*56 + 256*192 + 128*72 = 65536 = 512 x 128
 constexpr float RESCALE_THRESHOLD = 8.0f;  // log2 units: P may grow to 2^8 before O is rescaled
-#ifndef AKI_FWD_HEADS_PER_GROUP
-#define AKI_FWD_HEADS_PER_GROUP 32
-#endif
-constexpr int HEADS_PER_GROUP = AKI_FWD_HEADS_PER_GROUP;
+constexpr int HEADS_PER_GROUP = 32;        // (batch, head) slices per item group (header comment)
 }  // namespace fwd
 
 struct FwdKernelParams {
@@ -80,9 +70,9 @@ struct FwdKernelParams {
   int plan_pairs;
   int B, H, T;
   int q_off;             // queries are key rows [q_off, q_off + T) (AkiMmaAttnParams.q_offset)
-  int ranks, group, n_items, use_clc;   // items: ((g * ranks + r) * group + slice)
+  int ranks, group;      // items: ((g * ranks + r) * group + slice); the grid has one CTA per item
   float scale_log2, scale;
-  unsigned long long* trace;  // debug build (make TRACE=1, tools/fwd_trace.py): clock64 stamps of one CTA's first item
+  unsigned long long* trace;  // trace build (-DAKI_FWD_TRACE, tools/fwd_trace.py): clock64 stamps of one CTA's first item
   int trace_cta;
 };
 
@@ -114,30 +104,6 @@ __device__ __forceinline__ void umma_ts_lh(uint32_t d_tmem, uint32_t a_tmem, uin
       "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], db, %4, p;\n\t}\n" ::"r"(d_tmem),
       "r"(a_tmem), "r"(b_lo), "r"(desc_hi), "r"(idesc), "r"(accumulate)
       : "memory");
-}
-
-// exp2 of two scores on the FMA pipe (Cody-Waite split + degree-3 minimax polynomial, relative error 7.5e-5 -- far
-// below the bf16 rounding of P): x = n + f with n = round(x) taken from the mantissa of x + 1.5*2^23, 2^f from the
-// polynomial on [-0.5, 0.5], 2^n by adding n to the exponent field.  The MUFU unit (4 lanes per sub-partition) is the
-// scarcest pipe of this kernel (16 384 exponentials per 128 x 128 tile = 1024 cycles against ~1000 of tensor time), so
-// a share of the scores goes this way.  Inputs below -126 (masked scores are -inf) are clamped: they come out as
-// 2^-126 ~ 1e-38 instead of 0, which vanishes against the row maximum's 2^0.
-__device__ __forceinline__ void exp2_poly_x2(uint64_t a2, float& p0, float& p1) {
-  float a0, a1;
-  f32x2_unpack(a2, a0, a1);
-  a0 = fmaxf(a0, -126.f); a1 = fmaxf(a1, -126.f);
-  a2 = f32x2_pack(a0, a1);
-  const uint64_t t2 = f32x2_add(a2, f32x2_pack(12582912.f, 12582912.f));
-  const uint64_t n2 = f32x2_add(t2, f32x2_pack(-12582912.f, -12582912.f));
-  const uint64_t f2 = f32x2_fma(n2, f32x2_pack(-1.f, -1.f), a2);
-  uint64_t q = f32x2_fma(f2, f32x2_pack(0.0551716685f, 0.0551716685f), f32x2_pack(0.242611125f, 0.242611125f));
-  q = f32x2_fma(q, f2, f32x2_pack(0.693260968f, 0.693260968f));
-  q = f32x2_fma(q, f2, f32x2_pack(0.999928057f, 0.999928057f));
-  float q0, q1, t0, t1;
-  f32x2_unpack(q, q0, q1);
-  f32x2_unpack(t2, t0, t1);
-  p0 = __uint_as_float(__float_as_uint(q0) + (__float_as_uint(t0) << 23));
-  p1 = __uint_as_float(__float_as_uint(q1) + (__float_as_uint(t1) << 23));
 }
 
 // Rare path of the online softmax: the running max grew by more than the threshold, this thread's row of O_t is
@@ -328,11 +294,6 @@ attn_fwd_sm100_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_co
             publish(make_int4(1, b, h, len), make_int4(e.x, e.y, e.z >> 16, e.w >> 16),
                     make_int4(nk0, nk1, min(first_bad, (P.q_off + e.x + 1) / BN), min(first_bad, (P.q_off + e.y + 1) / BN)));
           }
-        }
-        if (!P.use_clc) {
-          id += gridDim.x;
-          if (id >= P.n_items) break;
-          continue;
         }
         mbar_arrive_expect_tx(BAR(CLC_BAR), 16);
         clc_try_cancel(smem_u32(&clc_resp), BAR(CLC_BAR));
@@ -543,14 +504,9 @@ attn_fwd_sm100_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_co
 #pragma unroll
           for (int x = 0; x < 32; ++x) {
             const uint64_t a2 = f32x2_fma(f32x2_pack(s[off + 2 * x], s[off + 2 * x + 1]), sc2, nm2);
-            float p0, p1;
-            if ((x & 3) >= 4 - AKI_FWD_POLY) {
-              exp2_poly_x2(a2, p0, p1);
-            } else {
-              float a0, a1;
-              f32x2_unpack(a2, a0, a1);
-              p0 = ex2_approx(a0); p1 = ex2_approx(a1);
-            }
+            float a0, a1;
+            f32x2_unpack(a2, a0, a1);
+            const float p0 = ex2_approx(a0), p1 = ex2_approx(a1);
             if (x & 1) sum_b = f32x2_add(sum_b, f32x2_pack(p0, p1));
             else sum_a = f32x2_add(sum_a, f32x2_pack(p0, p1));
             s[off + x] = __uint_as_float(pack_bf16x2(p0, p1));
@@ -654,8 +610,8 @@ attn_fwd_sm100_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_co
           ++n_od[t];
           tc_fence_after();
         }
-        // rows with no visible key (batch padding, keys all invalid): zeros (DESIGN.md).  Their maximum never left -inf;
-        // the row sum alone does not tell (the polynomial exp2 returns 2^-126, not 0, for a masked score)
+        // rows with no visible key (batch padding, keys all invalid): zeros (DESIGN.md).  Such a row's maximum never
+        // left -inf and its row sum stayed 0 (ex2 of a masked score is 0); either test tells, both are kept
         const float inv_l = (nk > 0 && i < len && lm.x > 0.f && lm.y > -INFINITY) ? 1.f / lm.x : 0.f;
         const bool store_row = (r < rows) && (ql < P.T);
         __nv_bfloat16* orow = P.o.row(b, store_row ? ql : 0, h);
@@ -771,15 +727,14 @@ int make_row_stats_map(CUtensorMap* m, void* base, int B, int H, int t_pad) {
   return AKI_OK;
 }
 
-// Per-device one-time setup (kernel attribute, SM count): the library may drive several GPUs from one process.
+// Per-device one-time setup (kernel attribute): the library may drive several GPUs from one process.
 struct FwdDeviceState {
   std::once_flag once;
-  int sm_count = 0;
   cudaError_t err = cudaSuccess;
 };
 static FwdDeviceState g_fwd_dev[64];
 
-static int fwd_device_setup(int* sm_count) {
+static int fwd_device_setup() {
   int dev = 0;
   if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) { set_last_cuda_error("cudaGetDevice failed"); return AKI_ERR_CUDA; }
   FwdDeviceState& s = g_fwd_dev[dev];
@@ -787,10 +742,8 @@ static int fwd_device_setup(int* sm_count) {
     s.err = cudaFuncSetAttribute(attn_fwd_sm100_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, fwd::SMEM_ALLOC);
     if (s.err == cudaSuccess)
       s.err = cudaFuncSetAttribute(attn_fwd_sm100_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, fwd::SMEM_ALLOC);
-    if (s.err == cudaSuccess) s.err = cudaDeviceGetAttribute(&s.sm_count, cudaDevAttrMultiProcessorCount, dev);
   });
   if (s.err != cudaSuccess) { set_last_cuda_error(cudaGetErrorString(s.err)); return AKI_ERR_CUDA; }
-  *sm_count = s.sm_count;
   return AKI_OK;
 }
 
@@ -823,12 +776,12 @@ extern "C" int aki_mma_attn_fwd(const AkiMmaAttnParams* p, aki_stream_t stream) 
   const long long n_groups = (slices + kp.group - 1) / kp.group;
   const long long n_items = n_groups * kp.ranks * kp.group;
   AKI_REQUIRE(n_items > 0 && n_items < (1ll << 31), AKI_ERR_BAD_SHAPE);
-  kp.n_items = (int)n_items;
   kp.scale = p->scale;
   kp.scale_log2 = p->scale * 1.4426950408889634f;
   kp.trace = nullptr; kp.trace_cta = -1;
 #ifdef AKI_FWD_TRACE
-  // Debug build only (make TRACE=1; tools/fwd_trace.py): dumps clock64 stamps of one CTA's first item and SYNCHRONISES.
+  // Trace build only (tools/build_variant.sh trace -DAKI_FWD_TRACE; tools/fwd_trace.py): dumps clock64 stamps of one
+  // CTA's first item and SYNCHRONISES.
   const char* trace_env = getenv("AKI_MMA_FWD_TRACE");
   const size_t trace_bytes = 4 * 64 * 12 * sizeof(unsigned long long);
   if (trace_env) {
@@ -837,12 +790,8 @@ extern "C" int aki_mma_attn_fwd(const AkiMmaAttnParams* p, aki_stream_t stream) 
     cudaMemset(kp.trace, 0, trace_bytes);
   }
 #endif
-  int sm_count = 0;
-  if ((rc = fwd_device_setup(&sm_count))) return rc;
-  // AKI_MMA_FWD_SCHED=static: persistent CTAs walk the items with a fixed stride instead of the hardware queue (A/B only)
-  static const bool use_static = []() { const char* e = getenv("AKI_MMA_FWD_SCHED"); return e && e[0] == 's'; }();
-  kp.use_clc = use_static ? 0 : 1;
-  const unsigned grid = kp.use_clc ? (unsigned)n_items : (unsigned)(n_items < sm_count ? n_items : sm_count);
+  if ((rc = fwd_device_setup())) return rc;
+  const unsigned grid = (unsigned)n_items;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   timing_hook_begin(st);
   if (p->rope_cos)

@@ -60,8 +60,8 @@ __device__ __forceinline__ bool mbar_test(uint32_t bar, uint32_t parity) {
 // completes (the default time limit is only ~80 cycles: a warp spinning on it issues ~1 instruction per 8 cycles and
 // hammers the MIO queue the MUFU instructions of the softmax warps go through -- ncu: a third of all warp instructions
 // of the forward kernel were such spins).  Release builds never trap: a kernel that is merely slowed down (profiler
-// replay, compute-sanitizer, MPS time slicing, a debugger) keeps waiting.  Bring-up builds (make TRAP=1 ->
-// -DAKI_MBAR_TRAP) turn a protocol bug into a CUDA error after AKI_MBAR_TRAP_NS of wall clock instead of hanging the box
+// replay, compute-sanitizer, MPS time slicing, a debugger) keeps waiting.  Bring-up builds
+// (tools/build_variant.sh trap -DAKI_MBAR_TRAP) turn a protocol bug into a CUDA error after AKI_MBAR_TRAP_NS of wall clock instead of hanging the box
 // (the hardware may return from try_wait long before the hint expires, so expired waits are not counted).
 #ifndef AKI_MBAR_TRAP_NS
 #define AKI_MBAR_TRAP_NS 4000000000ull   // bring-up builds: a wait longer than 4 s of wall clock is a protocol bug

@@ -11,7 +11,6 @@ Ops (torch.library, namespace ``aki_mma``):
 from __future__ import annotations
 
 import ctypes as C
-import os
 from dataclasses import dataclass
 from typing import Optional, Tuple
 
@@ -105,21 +104,15 @@ def rebuild_tile_bounds(s: MMASegments) -> MMASegments:
     return s
 
 
-PLAN_FLAGS = int(os.environ.get("AKI_MMA_PLAN_FLAGS", "3"))   # tools only: bit 0 cut at span starts, bit 1 rank + pair
-
-
-def build_fwd_plan(seq_len, row_lo, row_hi, vbits, T: int, max_spans: int = 8, flags: Optional[int] = None,
-                   q_offset: int = 0) -> torch.Tensor:
+def build_fwd_plan(seq_len, row_lo, row_hi, vbits, T: int, max_spans: int = 8, q_offset: int = 0) -> torch.Tensor:
     """Forward work plan (include/aki_mma.h, aki_mma_fwd_plan_at): (B, 1 + pairs, 4) int32 for the T query rows
     [q_offset, q_offset + T) of metadata in key coordinates."""
-    if not hasattr(lib, "aki_mma_fwd_plan"):      # AKI_MMA_LIB_COMPAT (tools): an ABI-1 build has no plan
-        return None
     B = seq_len.shape[0]
     nt = (T + TILE - 1) // TILE
     pairs = (nt + max_spans + 2) // 2
     plan = torch.empty(B, 1 + pairs, 4, dtype=torch.int32, device=seq_len.device)
     mp, bp = (row_lo.shape[1] if row_lo is not None else 0), (vbits.shape[1] if vbits is not None else 0)
-    fl = PLAN_FLAGS if flags is None else flags
+    fl = 3   # cut at span starts, rank and pair by key-tile count
     if q_offset:
         check(lib.aki_mma_fwd_plan_at(_ptr(seq_len), _ptr(row_lo), _ptr(row_hi), _ptr(vbits), B, T, int(q_offset), mp, bp,
                                       pairs, fl, _ptr(plan), _stream()), "aki_mma_fwd_plan_at")

@@ -1,15 +1,12 @@
 #!/bin/bash
-# Builds the current working tree into build/libaki_<name>.so (own object directory) for same-box A/B runs through
-# AKI_MMA_LIB (tools only).  usage: tools/build_variant.sh <name> [extra nvcc flags, e.g. -DAKI_FWD_TRACE]
+# Builds the current working tree into build/libaki_<name>.so from its own object directory, for same-box A/B runs
+# through AKI_MMA_LIB (tools only).  usage: tools/build_variant.sh <name> [extra nvcc flags]
+#   tools/build_variant.sh trace -DAKI_FWD_TRACE     clock64 stamps (tools/fwd_trace.py, tools/bwd_trace.py)
+#   tools/build_variant.sh trap -DAKI_MBAR_TRAP      a stuck mbarrier wait traps after 4 s (tools/stress.py)
+#   tools/build_variant.sh ko_red -DKO_RED           backward knockout (attn_bwd_sm100.cu): timing only, wrong results
 set -e
-name=$1; shift
+name=${1:?usage: tools/build_variant.sh <name> [extra nvcc flags]}; shift
 root=$(cd "$(dirname "$0")/.." && pwd)
-obj=$root/build/obj_$name
-mkdir -p $obj
-for f in api meta rope decode skinny_linear layer_elementwise attn_simt attn_fwd_sm100 attn_bwd_sm100; do
-  nvcc -gencode arch=compute_100a,code=sm_100a -O3 -std=c++17 -lineinfo -Xcompiler -fPIC --expt-relaxed-constexpr "$@" \
-    -c $root/aki_b200/csrc/$f.cu -o $obj/$f.o &
-done
-wait
-nvcc -gencode arch=compute_100a,code=sm_100a -shared -o $root/build/libaki_$name.so $obj/*.o -cudart static
-echo built $root/build/libaki_$name.so
+rm -rf "$root/build/obj_$name"
+make -C "$root/aki_b200/csrc" -j OBJ="$root/build/obj_$name" OUT="$root/build/libaki_$name.so" EXTRA="$*"
+echo built "$root/build/libaki_$name.so"

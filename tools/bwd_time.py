@@ -1,5 +1,5 @@
 """Kernel-only time of attn_bwd_sm100_kernel (T=8192, B=2, H=32; pure causal and 4 image spans) through the timing hook.
-Used with AKI_MMA_LIB=<variant> for same-box A/B and knockout runs (tools/build_bwd_ko.sh); no result check here."""
+Used with AKI_MMA_LIB=<variant> for same-box A/B and knockout runs (tools/build_variant.sh); no result check here."""
 import os, sys, statistics
 import numpy as np, torch
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
