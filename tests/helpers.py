@@ -219,3 +219,127 @@ def sum_eps(depth):
     """Relative error bound of an fp32 sum of non-negative terms in which every term passes through at most `depth`
     roundings (additions, or the rounding of an FMA that adds it): depth * 2^-24, to first order."""
     return depth * U32
+
+
+# ------------------------------------------------------------------------------------------------------------------
+# Visibility census (test_gpu_attention_census.py): with K = 0 every score is 0, so every visible key weighs exactly 1
+# and a one-hot V window (forward, decode) or a one-hot dO probe (backward) turns an output element into "does this
+# (row, key) pair attend": 1/n_i or bf16(P) where it does, exactly 0 where it does not.  The references below are plain
+# torch expressions of the oracle's predicate; they run on the device their tensors live on and never read the
+# kernels' metadata tensors.
+CENSUS_W = 32 * 96          # keys (forward, decode) or rows (backward) one launch maps: H * D output columns
+
+
+class MaskRef:
+    """The visibility predicate of expand_segments_to_4d in key coordinates, for B samples of Tk keys:
+    allowed(i, j) = i < len & j < len & ((j <= i & valid[j]) | (row_lo[i] <= j < row_hi[i] & mutual[j])).
+    seq_len (B,), row_lo / row_hi (B, Tk) int64; valid / mutual (B, Tk) bool."""
+
+    def __init__(self, seq_len, valid, mutual, row_lo, row_hi):
+        self.seq_len, self.valid, self.mutual = seq_len.to(torch.int64), valid.bool(), mutual.bool()
+        self.row_lo, self.row_hi = row_lo.to(torch.int64), row_hi.to(torch.int64)
+
+    @property
+    def B(self):
+        return self.valid.shape[0]
+
+    @property
+    def Tk(self):
+        return self.valid.shape[1]
+
+    def to(self, device):
+        return MaskRef(*(x.to(device) for x in (self.seq_len, self.valid, self.mutual, self.row_lo, self.row_hi)))
+
+    @staticmethod
+    def from_segments(S, T=None, text_only=False):
+        """The oracle's Segments (segments_ref) cut or zero-padded to T keys; text_only: image rows see later text keys
+        only (expand_segments_to_4d's text_only)."""
+        T = S.seg.shape[1] if T is None else T
+        m = min(T, S.seg.shape[1])
+
+        def cut(a, fill, dtype):
+            out = torch.full((a.shape[0], T), fill, dtype=dtype)
+            out[:, :m] = torch.from_numpy(np.ascontiguousarray(a[:, :m])).to(dtype)
+            return out
+        valid = cut(S.valid, 0, torch.bool)
+        mutual = valid & (cut(S.seg, -1, torch.int64) == 0) if text_only else valid
+        return MaskRef(torch.from_numpy(S.seq_len.astype(np.int64)), valid, mutual, cut(S.row_lo, 0, torch.int64),
+                       cut(S.row_hi, 0, torch.int64))
+
+    @staticmethod
+    def causal(B, T, seq_len=None):
+        """No metadata: every key up to the row (seq_len None = T for every sample)."""
+        sl = torch.full((B,), T, dtype=torch.int64) if seq_len is None else torch.as_tensor(seq_len, dtype=torch.int64)
+        ones = torch.ones(B, T, dtype=torch.bool)
+        zero = torch.zeros(B, T, dtype=torch.int64)
+        return MaskRef(sl, ones, ones, zero, zero)
+
+
+def allowed_slab(R, rows, cols):
+    """(B, r1 - r0, c1 - c0) bool: allowed(i, j) for rows i in range(*rows), keys j in range(*cols), key coordinates.
+    Rows and keys at or beyond Tk see / are seen by nothing."""
+    (r0, r1), (c0, c1) = rows, cols
+    dev = R.valid.device
+    i = torch.arange(r0, r1, device=dev)[None, :, None]
+    j = torch.arange(c0, c1, device=dev)[None, None, :]
+    ic, jc = i.clamp(max=R.Tk - 1)[0, :, 0], j.clamp(max=R.Tk - 1)[0, 0]
+    n = torch.minimum(R.seq_len, torch.tensor(R.Tk, device=dev))[:, None, None]
+    valid, mutual = R.valid[:, jc][:, None, :], R.mutual[:, jc][:, None, :]
+    lo, hi = R.row_lo[:, ic][:, :, None], R.row_hi[:, ic][:, :, None]
+    ok = ((j <= i) & valid) | ((j >= lo) & (j < hi) & mutual)
+    return ok & (i < n) & (j < n)
+
+
+def visible_counts(R):
+    """(B, Tk) int64: number of keys each row sees (row sums of allowed), from prefix sums, not from allowed_slab."""
+    dev = R.valid.device
+    i = torch.arange(R.Tk, device=dev)[None]
+    n = torch.minimum(R.seq_len, torch.tensor(R.Tk, device=dev))[:, None]
+    z = torch.zeros(R.B, 1, dtype=torch.int64, device=dev)
+    cv = torch.cat([z, (R.valid & (i < n)).to(torch.int64).cumsum(1)], 1)       # cv[k] = valid keys among [0, k)
+    cm = torch.cat([z, (R.mutual & (i < n)).to(torch.int64).cumsum(1)], 1)
+    causal = cv.gather(1, (i + 1).clamp(max=R.Tk).expand(R.B, -1))
+    lo = torch.maximum(R.row_lo, i + 1).clamp(min=0).minimum(n)                  # keys after the row: not counted twice
+    hi = R.row_hi.clamp(min=0).minimum(n)
+    ext = torch.where(hi > lo, cm.gather(1, hi) - cm.gather(1, lo.minimum(hi)), torch.zeros_like(hi))
+    return torch.where(i < n, causal + ext, torch.zeros_like(causal))
+
+
+def decode_visible(kv_len, kv_start, valid, n_keys):
+    """(B, n_keys) bool: the keys a decode query attends, kv_start[b] <= j < kv_len[b] and valid[b, j] (kv_start /
+    valid None: 0 / every key)."""
+    kv_len = torch.as_tensor(kv_len, dtype=torch.int64)
+    j = torch.arange(n_keys, device=kv_len.device)[None]
+    vis = j < kv_len[:, None]
+    if kv_start is not None:
+        vis &= j >= torch.as_tensor(kv_start, dtype=torch.int64, device=kv_len.device)[:, None]
+    if valid is not None:
+        vis &= valid[:, :n_keys].to(kv_len.device).bool()
+    return vis
+
+
+def recip_bf16(n):
+    """bf16(fp32(1 / n)) as fp64 for integer counts n >= 1 (0 where n == 0): what a kernel writes for a visible key
+    when every visible key weighs exactly 1 (fp32 IEEE division, one bf16 rounding)."""
+    nf = n.to(torch.float32)
+    r = torch.where(n > 0, 1.0 / nf.clamp(min=1), torch.zeros_like(nf))
+    return r.to(torch.bfloat16).to(torch.float64)
+
+
+def census_diff(got, want, rows, keys):
+    """Pairs where the kernel's map (got != 0) and the reference map `want` disagree: (K, 5) float64 rows
+    (b, row, key, got, want), sorted.  got / want are (B, len(rows), len(keys)); rows / keys the key-coordinate indices
+    of those axes."""
+    bad = (got != 0) != want
+    idx = bad.nonzero()
+    if idx.numel() == 0:
+        return torch.zeros(0, 5, dtype=torch.float64)
+    b, r, k = idx.unbind(1)                                           # nonzero() is in (b, row, key) order
+    return torch.stack([b.double(), rows.to(idx.device)[r].double(), keys.to(idx.device)[k].double(),
+                        got[b, r, k].double(), want[b, r, k].double()], 1).cpu()
+
+
+def census_message(diff, what):
+    b, r, k, g, w = diff[0].tolist()
+    return (f"{what}: {diff.shape[0]} (row, key) pairs attended wrongly; first (b, row, key, got, want) = "
+            f"({int(b)}, {int(r)}, {int(k)}, {g:.6g}, {bool(w)})")
